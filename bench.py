@@ -54,7 +54,11 @@ def parse():
     ap.add_argument("--knn-rows", type=int, default=10_000_000, help="rows of the descriptor map of the Hamming leg (0 = skip)")
     ap.add_argument("--proj-points", type=int, default=500_000, help="map points of the ProjectionMatch leg (0 = skip)")
     ap.add_argument("--clock-period", type=float, default=0.05, help="seconds between NVML clock samples (0 = no sampling)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
 
 
 def make_frames(n):
@@ -66,6 +70,30 @@ def make_frames(n):
         Ls.append(l)
         Rs.append(r)
     return np.concatenate(Ls), np.concatenate(Rs)
+
+
+def dump_outputs(path, d_out, F, cap, n_frames=32):
+    """What the caller of sfe_stereo_sequence_dev receives from one step, for a fixed sample of its frames
+    (default_rng(0); 32 of 128 frames are about 27 MB): keypoint fields, descriptor bytes, keypoint counts, stereo and
+    tracking indices and distances, one DIR/<name>.npy each, float32 (every value is exact in it).  Slots past a frame's
+    keypoint count hold no result and are written as 0."""
+    from slam_toolkit_b200 import api
+    frames = np.sort(np.random.default_rng(0).choice(F, min(F, n_frames), replace=False))
+    n = {s: d_out[f"n_{s}"].download((F,), np.int32)[frames] for s in "lr"}
+    valid = {s: np.arange(cap)[None, :] < n[s][:, None] for s in "lr"}
+    arrays = {"frames": frames, "n_l": n["l"], "n_r": n["r"]}
+    for s in "lr":
+        kps = d_out[f"kps_{s}"].download((F, cap), api.KP_DTYPE)[frames]
+        for field in api.KP_DTYPE.names:
+            arrays[f"kps_{s}_{field}"] = np.where(valid[s], kps[field], 0)
+        arrays[f"desc_{s}"] = np.where(valid[s][..., None], d_out[f"desc_{s}"].download((F, cap, 32), np.uint8)[frames], 0)
+    for k in ("stereo_idx", "stereo_dist", "track_idx", "track_dist"):     # per left keypoint
+        arrays[k] = np.where(valid["l"], d_out[k].download((F, cap), np.int32)[frames], 0)
+    arrays = {k: a.astype(np.float32) for k, a in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
 
 
 def track_params():
@@ -439,6 +467,8 @@ def main():
     ex.wait()
     sampler.active = False
     ms = ev0.elapsed_ms(ev1)
+    if args.dump_outputs and rank == 0:     # before the extract-only leg below reuses the output buffers
+        dump_outputs(args.dump_outputs, d_out, F, cap)
     barrier()
     launches = ex.launches() - l0
     # BASELINE config 3 beside the headline: extraction only (sfe_extract_batch_dev) of the same resident images, 2F

@@ -7,7 +7,14 @@ src/orb_extractor.cpp:684, orders equal counts by creation = the oracle's declar
 tables, pyramid, the 19-px ring, FAST candidates, quadtree survivors and their order, angles, blurred planes,
 descriptors, StereoMatch, ProjectionMatch.  With glibc's heap the reference itself moves; there the test asserts equality
 on every level whose quadtree did NOT stop inside a group of equally-full nodes and reports the rest.
-CPU only; skipped when neither the prebuilt library nor /root/reference is present."""
+
+The reference's side of each comparison comes from oracle/_ref when that library is built (it needs the reference's
+sources, which are not part of this repository), else from tests/golden/ref_pinning.json: the SHA-256 of every array the
+reference returned here (and the quaternions its SE3Quat holds, which feed later calls).  With the library present
+every live value must also equal its recorded digest; SFE_RECORD_REF_PINS=1 rewrites the file from the live library
+instead.  Only the glibc-heap test needs the library itself.  CPU only."""
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -16,16 +23,78 @@ import pytest
 from slam_toolkit_b200 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+PINS = os.path.join(ROOT, "tests", "golden", "ref_pinning.json")
+
+
+def _digest(a):
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype.str}{a.shape}".encode() + a.tobytes()).hexdigest()[:32]
+
+
+class Pins:
+    """The reference's side of the comparisons of one test: `ref` is the live oracle/_ref binding or None."""
+
+    def __init__(self, ref, stored, record, test):
+        self.ref, self.stored, self.record, self.test = ref, stored, record, test
+
+    def _key(self, key):
+        return f"{self.test}/{key}"
+
+    def equal(self, key, got, want):
+        """got (the oracle's value) equals want() (the reference's), byte for byte"""
+        k = self._key(key)
+        got = np.asarray(got)
+        if self.ref is None:
+            assert k in self.stored["digests"], f"no recorded reference value for {k}"
+            assert _digest(got) == self.stored["digests"][k], k
+            return
+        w = np.asarray(want())
+        assert got.dtype == w.dtype and got.shape == w.shape and got.tobytes() == w.tobytes(), k
+        if self.record:
+            self.stored["digests"][k] = _digest(w)
+        else:
+            assert self.stored["digests"].get(k) == _digest(w), f"{k}: the live reference differs from its recorded digest"
+
+    def value(self, key, want):
+        """a float64 vector the reference computed (used as an input of later calls)"""
+        k = self._key(key)
+        if self.ref is None:
+            return np.array(self.stored["values"][k], np.float64)
+        w = np.asarray(want(), np.float64)
+        if self.record:
+            self.stored["values"][k] = w.tolist()
+        else:
+            assert np.array_equal(np.array(self.stored["values"].get(k, []), np.float64).view(np.uint64), w.view(np.uint64)), k
+        return w
 
 
 @pytest.fixture(scope="module")
-def ref():
+def pins_store():
     import ref_c
-    if not ref_c.available():
-        pytest.skip("oracle/_ref is not built and the reference sources are absent")
-    ref_c.set_heap_mode(ref_c.HEAP_MONOTONIC)
-    yield ref_c
-    ref_c.set_heap_mode(ref_c.HEAP_MONOTONIC)
+    live = ref_c if ref_c.available() else None
+    record = live is not None and os.environ.get("SFE_RECORD_REF_PINS") == "1"
+    if record:
+        stored = {"digests": {}, "values": {}}
+    else:
+        with open(PINS) as f:
+            stored = json.load(f)
+    if live is not None:
+        live.set_heap_mode(live.HEAP_MONOTONIC)
+    yield live, stored, record
+    if live is not None:
+        live.set_heap_mode(live.HEAP_MONOTONIC)
+    if record:
+        stored["generator"] = ("oracle/_ref: the reference's own src/orb_extractor.cpp, src/matcher.cpp, src/camera.cpp compiled "
+                               "unmodified (oracle/ref_build), monotonic heap; written by SFE_RECORD_REF_PINS=1 pytest "
+                               "tests/test_ref_pinning.py")
+        with open(PINS, "w") as f:
+            json.dump(stored, f, indent=0, sort_keys=True)
+
+
+@pytest.fixture
+def pin(pins_store, request):
+    live, stored, record = pins_store
+    return Pins(live, stored, record, request.node.name)
 
 
 def _cam(oracle, d=(0, 0, 0, 0), w=synth.KITTI_W, h=synth.KITTI_H):
@@ -36,79 +105,88 @@ def _reflect101_ring(img, e=19):
     return np.pad(img, e, mode="reflect")
 
 
-def _compare_extraction(oracle, ref, o, r, img):
+def _or_empty(plane):
+    return np.zeros(0, np.int8) if plane is None else plane
+
+
+def _compare_extraction(oracle, pin, o, r, img, tag):
+    """o: oracle extractor; r: the reference's extractor with the same parameters (None without the library)"""
     ko, do = o.extract(img)
-    kr, dr = r.extract(img)
+    if r is not None:
+        kr, dr = r.extract(img)
     for l in range(o.nlevels):
         lo = o.level(l)
-        assert np.array_equal(lo, r.level(l)), f"pyramid level {l}"
-        assert np.array_equal(_reflect101_ring(lo), r.level(l, ring=True)), f"reflected ring of level {l}"
-        co, cr = o.candidates(l), r.candidates(l)
-        assert co.shape == cr.shape and np.array_equal(co, cr), f"FAST candidates level {l} (set and order)"
-        w, h = r.level_size(l)
+        pin.equal(f"{tag}/level{l}", lo, lambda: r.level(l))
+        pin.equal(f"{tag}/ring{l}", _reflect101_ring(lo), lambda: r.level(l, ring=True))
+        co = o.candidates(l)
+        pin.equal(f"{tag}/candidates{l}", co, lambda: r.candidates(l))       # set and order
         if len(co):
             quota = int(o.tables()["per_level"][l])
-            assert np.array_equal(o.distributed(l), r.distribute(co, 16, w - 16, 16, h - 16, quota, l)), f"quadtree level {l}"
-        rb = r.blur(l)
-        if rb is not None:
-            assert np.array_equal(o.blur(l), rb), f"blurred level {l}"
-        else:
+            h, w = lo.shape
+            pin.equal(f"{tag}/quadtree{l}", o.distributed(l), lambda: r.distribute(co, 16, w - 16, 16, h - 16, quota, l))
+        ob = o.blur(l)
+        pin.equal(f"{tag}/blur{l}", _or_empty(ob), lambda: _or_empty(r.blur(l)))   # only levels that kept keypoints are blurred
+        if ob is None:
             assert len(o.distributed(l)) == 0
-    assert len(ko) == len(kr)
     for f in ko.dtype.names:  # angle compared by bits: fastAtan2 output
-        assert np.array_equal(ko[f].view(np.uint32), kr[f].view(np.uint32)), f"keypoint field {f}"
-    assert np.array_equal(do, dr), "descriptors"
+        pin.equal(f"{tag}/kp.{f}", ko[f], lambda: kr[f])
+    pin.equal(f"{tag}/descriptors", do, lambda: dr)
     return ko, do
 
 
-def test_ctor_tables_equal_the_reference(oracle, ref):
+def _ref_extractor(pin, *params):
+    return pin.ref.Extractor(*params) if pin.ref is not None else None
+
+
+def test_ctor_tables_equal_the_reference(oracle, pin):
     for nf, sf, nl in [(2000, 1.2, 8), (500, 1.2, 4), (300, 1.5, 3), (1000, 1.2, 8), (50, 1.2, 2), (20, 1.2, 8), (1500, 1.1, 12),
                        (4000, 2.0, 5), (1, 1.2, 8), (777, 1.33, 7)]:
-        to, tr = oracle.Extractor(nf, sf, nl, 20, 7).tables(), ref.Extractor(nf, sf, nl, 20, 7).tables()
+        to = oracle.Extractor(nf, sf, nl, 20, 7).tables()
+        tr = _ref_extractor(pin, nf, sf, nl, 20, 7)
         for k in to:
-            assert np.array_equal(to[k].view(np.uint32), tr[k].view(np.uint32)), (k, nf, sf, nl)
+            pin.equal(f"{nf},{sf},{nl}/{k}", to[k], lambda: tr.tables()[k])
 
 
 @pytest.mark.parametrize("seed", range(8))
-def test_kitti_frames_every_stage(oracle, ref, seed):
-    o, r = oracle.Extractor(), ref.Extractor()
+def test_kitti_frames_every_stage(oracle, pin, seed):
+    o, r = oracle.Extractor(), _ref_extractor(pin)
     L, R = synth.stereo_pair(seed)
-    kl, dl = _compare_extraction(oracle, ref, o, r, L)
-    kr, dr = _compare_extraction(oracle, ref, o, r, R)
+    kl, dl = _compare_extraction(oracle, pin, o, r, L, "L")
+    kr, dr = _compare_extraction(oracle, pin, o, r, R, "R")
     si, _ = oracle.stereo_match(kl, dl, kr, dr)
-    assert np.array_equal(si, ref.stereo_match(kl, dl, kr, dr, _cam(oracle)))
+    pin.equal("stereo", si, lambda: pin.ref.stereo_match(kl, dl, kr, dr, _cam(oracle)))
     assert (si >= 0).sum() > 1000
 
 
 @pytest.mark.parametrize("case", [(320, 240, 500, 1.2, 4, 20, 7), (161, 131, 300, 1.5, 3, 20, 7), (640, 200, 1000, 1.2, 8, 30, 10),
                                   (97, 95, 50, 1.2, 2, 20, 7), (1241, 376, 20, 1.2, 8, 20, 7), (800, 600, 3000, 1.2, 8, 20, 7),
                                   (333, 500, 700, 1.3, 6, 25, 5), (1920, 1080, 2000, 1.2, 8, 20, 7)])
-def test_other_geometries(oracle, ref, case):
+def test_other_geometries(oracle, pin, case):
     w, h, nf, sf, nl, it, mt = case
     img, _ = synth.stereo_pair(100 + w % 7, w, h)
-    _compare_extraction(oracle, ref, oracle.Extractor(nf, sf, nl, it, mt), ref.Extractor(nf, sf, nl, it, mt), img)
+    _compare_extraction(oracle, pin, oracle.Extractor(nf, sf, nl, it, mt), _ref_extractor(pin, nf, sf, nl, it, mt), img, "img")
 
 
-def test_noise_flat_and_retry_images(oracle, ref):
+def test_noise_flat_and_retry_images(oracle, pin):
     """noise (every level far over quota, very long careful phase), flat (nothing), low contrast (20 -> 7 retry)"""
     rng = np.random.default_rng(3)
-    o, r = oracle.Extractor(), ref.Extractor()
+    o, r = oracle.Extractor(), _ref_extractor(pin)
     noise = rng.integers(0, 256, (376, 1241), dtype=np.uint8)
-    k, _ = _compare_extraction(oracle, ref, o, r, noise)
+    k, _ = _compare_extraction(oracle, pin, o, r, noise, "noise")
     assert len(k) >= 2000
-    k, _ = _compare_extraction(oracle, ref, o, r, np.full((376, 1241), 77, np.uint8))
+    k, _ = _compare_extraction(oracle, pin, o, r, np.full((376, 1241), 77, np.uint8), "flat")
     assert len(k) == 0
     soft = (synth.stereo_pair(11)[0].astype(np.float32) * 0.12 + 100).astype(np.uint8)   # contrast below iniThFAST
-    k, _ = _compare_extraction(oracle, ref, o, r, soft)
+    k, _ = _compare_extraction(oracle, pin, o, r, soft, "soft")
     assert len(k) > 0
     mixed = synth.stereo_pair(12)[0].copy()
     mixed[:, 600:] = (mixed[:, 600:].astype(np.float32) * 0.1 + 90).astype(np.uint8)
-    _compare_extraction(oracle, ref, o, r, mixed)
+    _compare_extraction(oracle, pin, o, r, mixed, "mixed")
 
 
-def test_distribute_random_candidate_sets(oracle, ref):
+def test_distribute_random_candidate_sets(oracle, pin):
     """DistributeOctTree + DivideNode (src/orb_extractor.cpp:481-763) on synthetic candidate lists with many equal counts"""
-    r = ref.Extractor()
+    r = _ref_extractor(pin)
     rng = np.random.default_rng(5)
     for t in range(60):
         W, H = int(rng.integers(40, 1300)), int(rng.integers(40, 500))
@@ -124,13 +202,15 @@ def test_distribute_random_candidate_sets(oracle, ref):
         xyr = np.stack([xs, ys, resp], 1)
         want = int(rng.integers(1, 2500))
         a = oracle.distribute(xyr, 16, 16 + W, 16, 16 + H, want)
-        b = r.distribute(xyr, 16, 16 + W, 16, 16 + H, want)
-        assert np.array_equal(a, b), (t, W, H, n, want)
+        pin.equal(f"{t}", a, lambda: r.distribute(xyr, 16, 16 + W, 16, 16 + H, want))
 
 
-def test_glibc_heap_moves_only_levels_cut_inside_a_tie_group(oracle, ref):
+def test_glibc_heap_moves_only_levels_cut_inside_a_tie_group(oracle, pin):
     """The reference as it runs on this machine (glibc malloc): equal to the oracle as a SET on every level whose careful
     phase did not stop between two equally-full nodes; the others are where the heap-address order decides (T1)."""
+    if pin.ref is None:
+        pytest.skip("glibc's heap order is the live reference library's own, and oracle/_ref is not built")
+    ref = pin.ref
     o, r = oracle.Extractor(), ref.Extractor()
     total = moved = cut_levels = levels = 0
     for seed in range(8):
@@ -153,14 +233,15 @@ def test_glibc_heap_moves_only_levels_cut_inside_a_tie_group(oracle, ref):
     assert moved < 0.05 * total
 
 
-def test_descriptor_distance_and_atan2(oracle, ref):
+def test_descriptor_distance_and_atan2(oracle, pin):
     rng = np.random.default_rng(9)
     d = rng.integers(0, 256, (300, 32), dtype=np.uint8)
-    for i in range(0, 300, 2):
-        assert oracle.hamming256(d[i], d[i + 1]) == ref.hamming256(d[i], d[i + 1]) == int(np.unpackbits(d[i] ^ d[i + 1]).sum())
+    got = np.array([oracle.hamming256(d[i], d[i + 1]) for i in range(0, 300, 2)], np.int32)
+    assert np.array_equal(got, [int(np.unpackbits(d[i] ^ d[i + 1]).sum()) for i in range(0, 300, 2)])
+    pin.equal("hamming", got, lambda: np.array([pin.ref.hamming256(d[i], d[i + 1]) for i in range(0, 300, 2)], np.int32))
 
 
-def test_se3_and_camera_primitives(oracle, ref):
+def test_se3_and_camera_primitives(oracle, pin):
     """predicted_Tcw * Xw (g2o::SE3Quat, quaternion product), Camera::Project / IsInImage / NormalizedUndistort by bits"""
     rng = np.random.default_rng(0)
     for t in range(100):
@@ -170,14 +251,14 @@ def test_se3_and_camera_primitives(oracle, ref):
             q = np.array([0, 0, 0, 1.0]) + rng.normal(size=4) * 1e-2
         qt = np.concatenate([q, rng.normal(size=3)])
         x = rng.normal(size=(300, 3)) * rng.uniform(0.1, 100)
-        yr, qh = ref.se3_apply(qt, x)
+        qh = pin.value(f"{t}/q", lambda: pin.ref.se3_apply(qt, x)[1])
         assert abs(np.linalg.norm(qh) - 1) < 1e-15 and qh[3] >= 0
         yo = oracle.se3_apply(np.concatenate([qh, qt[4:]]), x)
-        assert np.array_equal(yr.view(np.uint64), yo.view(np.uint64))
+        pin.equal(f"{t}/xc", yo, lambda: pin.ref.se3_apply(qt, x)[0])
     cam = _cam(oracle, (-0.1, 0.02, 0.001, -0.0005))
     kps = np.zeros(500, oracle.KP_DTYPE)
     kps["x"], kps["y"] = rng.uniform(0, 1241, 500), rng.uniform(0, 376, 500)
-    assert np.array_equal(oracle.normalized_undistort(cam, kps).view(np.uint64), ref.normalized_undistort(cam, kps).view(np.uint64))
+    pin.equal("undistort", oracle.normalized_undistort(cam, kps), lambda: pin.ref.normalized_undistort(cam, kps))
 
 
 def _projection_inputs(seed, kl, dl, n=3000):
@@ -200,26 +281,30 @@ def _projection_inputs(seed, kl, dl, n=3000):
 
 
 @pytest.mark.parametrize("seed", range(3))
-def test_projection_match_equals_the_reference(oracle, ref, seed):
-    r = ref.Extractor()
-    kl, dl = r.extract(synth.stereo_pair(seed)[0])
+def test_projection_match_equals_the_reference(oracle, pin, seed):
+    img = synth.stereo_pair(seed)[0]
+    kl, dl = oracle.Extractor().extract(img)          # the frame: the reference's keypoints, pinned right here
+    r = _ref_extractor(pin)
+    if r is not None:
+        kr, dr = r.extract(img)
+    pin.equal("kps", kl, lambda: kr)
+    pin.equal("desc", dl, lambda: dr)
     xw, md, skip = _projection_inputs(seed, kl, dl)
     for d4 in ((0, 0, 0, 0), (-0.1, 0.02, 0.001, -0.0005)):
         cam = _cam(oracle, d4)
         for qt_in in ([0, 0, 0, 1, 0, 0, 0], [0.01, -0.02, 0.005, 0.9997, 0.1, -0.05, 0.2], [0.3, -0.1, 0.2, -0.9, 1.0, 0.5, 4.0]):
-            _, q = ref.se3_apply(np.array(qt_in, float), xw[:1])
+            q = pin.value(f"{qt_in}/q", lambda: pin.ref.se3_apply(np.array(qt_in, float), xw[:1])[1])
             qt = np.concatenate([q, np.array(qt_in[4:], float)])
             for radius in (50.0, 10.0, 100.0):
-                want = ref.projection_match(xw, md, skip, qt, cam, kl, dl, radius)
                 for grid in (False, True):
                     got, dist = oracle.projection_match(xw, md, skip, qt, cam, kl, dl, radius, grid=grid)
-                    assert np.array_equal(got, want), (d4, qt_in, radius, grid)
+                    pin.equal(f"{d4}/{qt_in}/{radius}", got, lambda: pin.ref.projection_match(xw, md, skip, qt, cam, kl, dl, radius))
                     ok = got >= 0
                     assert all(dist[j] == oracle.hamming256(md[got[j]], dl[j]) for j in np.nonzero(ok)[0])
 
 
 def test_projection_golden_fixture(oracle):
-    """the committed ProjectionMatch result of the reference (tools/gen_golden.py) -- runs without _ref (GPU box)"""
+    """the committed ProjectionMatch result of the reference (tools/gen_golden.py)"""
     z = np.load(os.path.join(ROOT, "tests/golden/golden_proj.npz"))
     g = np.load(os.path.join(ROOT, "tests/golden/golden_seed0.npz"))
     cam = _cam(oracle, z["dist4"])
@@ -230,7 +315,7 @@ def test_projection_golden_fixture(oracle):
         assert (got >= 0).sum() > 10
 
 
-def test_stereo_match_edge_cases_equal_the_reference(oracle, ref):
+def test_stereo_match_edge_cases_equal_the_reference(oracle, pin):
     """hand-built rows: single candidate (accepted, dist1 = 999999999), tie for best (rejected), dy = +-3 exactly,
     dx = 0 / 100 / just outside, negative dx, bucket borders (y multiples of 10), an empty right set"""
     rng = np.random.default_rng(21)
@@ -250,4 +335,4 @@ def test_stereo_match_edge_cases_equal_the_reference(oracle, ref):
             dl[0] = dr[2]
             kr[2]["x"], kr[2]["y"] = kl[0]["x"], kl[0]["y"] - 3           # dx = 0, dy = 3
         got, _ = oracle.stereo_match(kl, dl, kr, dr)
-        assert np.array_equal(got, ref.stereo_match(kl, dl, kr, dr, cam)), trial
+        pin.equal(f"{trial}", got, lambda: pin.ref.stereo_match(kl, dl, kr, dr, cam))
