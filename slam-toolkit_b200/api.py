@@ -347,6 +347,14 @@ class ORBextractor:
     def _grow_cap(self, w, h):  # a very wide image can return more than the default bound: 4 * nIni nodes per level
         self.cap = max(self.cap, self.cap_for(w, h))
 
+    def _out_cap(self, cap, w, h) -> int:
+        """the row stride of caller-allocated output arrays: their own capacity, which must hold one w x h image's keypoints
+        (self.cap may have grown since they were allocated)"""
+        need = self.cap_for(w, h)
+        if cap < need:
+            raise SfeError(SFE_ERR_CAPACITY, f"out holds {cap} keypoints per image, a {w} x {h} image can return {need}")
+        return cap
+
     def close(self):
         if getattr(self, "h", None):
             lib().sfe_extractor_destroy(self.h)
@@ -413,8 +421,11 @@ class ORBextractor:
         if out is None:
             self._grow_cap(w, h)
             out = (np.zeros((count, self.cap), KP_DTYPE), np.zeros((count, self.cap, 32), np.uint8), np.zeros(count, np.int32))
+            cap = self.cap
+        else:
+            cap = self._out_cap(out[0].shape[1], w, h)
         kps, desc, n = out
-        _check(lib().sfe_extract_batch(self.h, _p(images), w * h, count, w, h, w, _p(kps), _p(desc), self.cap, _p(n)))
+        _check(lib().sfe_extract_batch(self.h, _p(images), w * h, count, w, h, w, _p(kps), _p(desc), cap, _p(n)))
         self._wh = (w, h)
         return kps, desc, n
 
@@ -433,10 +444,11 @@ class ORBextractor:
         if out is None:
             self._grow_cap(w, h)
             out = self.alloc_stereo_out(f)
+        cap = self._out_cap(out["kps_l"].shape[1], w, h)
         sp = C.byref(stereo_params) if stereo_params is not None else None
         _check(lib().sfe_stereo_frames(self.h, _p(left), _p(right), w * h, f, w, h, w, sp, _p(out["kps_l"]), _p(out["desc_l"]),
                                        _p(out["n_l"]), _p(out["kps_r"]), _p(out["desc_r"]), _p(out["n_r"]),
-                                       _p(out["stereo_idx"]), _p(out["stereo_dist"]), self.cap))
+                                       _p(out["stereo_idx"]), _p(out["stereo_dist"]), cap))
         self._wh = (w, h)
         return out
 
@@ -451,11 +463,12 @@ class ORBextractor:
         if out is None:
             self._grow_cap(w, h)
             out = self.alloc_stereo_out(f, track=True)
+        cap = self._out_cap(out["kps_l"].shape[1], w, h)
         sp = C.byref(stereo_params) if stereo_params is not None else None
         _check(lib().sfe_stereo_sequence(self.h, _p(left), _p(right), w * h, f, w, h, w, sp, C.byref(track_params),
                                          _p(out["kps_l"]), _p(out["desc_l"]), _p(out["n_l"]), _p(out["kps_r"]),
                                          _p(out["desc_r"]), _p(out["n_r"]), _p(out["stereo_idx"]), _p(out["stereo_dist"]),
-                                         _p(out["track_idx"]), _p(out["track_dist"]), self.cap))
+                                         _p(out["track_idx"]), _p(out["track_dist"]), cap))
         self._wh = (w, h)
         return out
 

@@ -24,6 +24,7 @@
 // Output = the same per-(chunk, query) pair of 64-bit keys (distance << 32 | global row) the other partial kernels
 // write, so knn2_merge_kernel / knn2_merge_push_kernel finish the job.
 #include <algorithm>
+#include <mutex>
 
 #include "sfe_common.cuh"
 #include "sfe_tma.cuh"
@@ -379,16 +380,17 @@ cudaError_t launch_knn2_unpack_tiles(cudaStream_t st, const uint8_t *db, long lo
 // ready-made operand tiles (launch_knn2_unpack_tiles), fetched by bulk copies instead of being unpacked by the producer warps.
 cudaError_t launch_knn2_tc(cudaStream_t st, int sm_count, const uint8_t *db, const uint8_t *tiles, long long rows, long long idx_base,
                            int chunk_rows, int chunks, const uint8_t *queries, int q, unsigned long long *part) {
-    static bool configured[64] = {};
+    static std::once_flag once[64];  // matchers of one device may search from several threads at once
+    static cudaError_t configured[64];
     int dev = 0;
     cudaGetDevice(&dev);
     const size_t smem = knn2_tc_smem_bytes(), smem_bulk = sizeof(TcSmemT<kBulkStages>) + 128;
-    if (!configured[dev & 63]) {
+    std::call_once(once[dev & 63], [&] {
         cudaError_t e = cudaFuncSetAttribute(knn2_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(knn2_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bulk);
-        if (e != cudaSuccess) return e;
-        configured[dev & 63] = true;
-    }
+        configured[dev & 63] = e;
+    });
+    if (configured[dev & 63] != cudaSuccess) return configured[dev & 63];
     const int groups = (q + kGroupQ - 1) / kGroupQ;
     const int grid = std::min(sm_count, groups * chunks);
     if (tiles)

@@ -1231,9 +1231,13 @@ struct sfe_db {
     uint8_t *rows_dev = nullptr;
     int64_t rows = 0, idx_base = 0;
     // the rows as ready-made int8 operand tiles of the tensor-core kernel (8 x the packed size), built at the first
-    // many-query search when the policy (knn_tiles_max_bytes) allows; tiles_tried: do not try again
+    // many-query search when the policy (knn_tiles_max_bytes) allows; tiles_tried: do not try again.  Every matcher of the
+    // device may search the database, from any thread: tiles_mu guards the build, which runs on the stream of the matcher
+    // that comes first, and tiles_ready (recorded behind the unpack) is what every search that reads the tiles waits for.
+    mutable std::mutex tiles_mu;
     mutable uint8_t *tiles_dev = nullptr;
     mutable bool tiles_tried = false;
+    mutable cudaEvent_t tiles_ready = nullptr;
 };
 
 // keys_out != nullptr: leave the per-keypoint (dist << 32 | ~global query) keys there (one shard's contribution to a
@@ -1351,21 +1355,39 @@ static int knn_partial(sfe_matcher *m, const sfe_db *db, const uint8_t *q_dev, i
         // A map that is searched with many queries keeps its rows unpacked in HBM (256 B per row instead of 32): the kernel's
         // producers then move tiles with bulk copies instead of unpacking 10 M rows once per query group.  Built on first use,
         // when it fits the budget (SFE_KNN_TILES_MAX_GB, default 16 GB and a quarter of the free memory).
-        if (!db->tiles_dev && !db->tiles_tried && q >= 256 && db->rows >= 65536) {
-            db->tiles_tried = true;
-            const size_t need = knn2_tc_tiles_bytes(db->rows);
-            size_t free_b = 0, total_b = 0;
-            if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need <= m->knn_tiles_max_bytes && need <= free_b / 4) {
-                if (cudaMalloc((void **)&db->tiles_dev, need) == cudaSuccess) {
-                    SFE_CUDA(launch_knn2_unpack_tiles(st, db->rows_dev, db->rows, db->tiles_dev));
+        const uint8_t *tiles = nullptr;
+        {
+            std::lock_guard<std::mutex> lock(db->tiles_mu);
+            if (!db->tiles_dev && !db->tiles_tried && q >= 256 && db->rows >= 65536) {
+                db->tiles_tried = true;
+                const size_t need = knn2_tc_tiles_bytes(db->rows);
+                size_t free_b = 0, total_b = 0;
+                uint8_t *t = nullptr;
+                if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need <= m->knn_tiles_max_bytes && need <= free_b / 4) {
+                    if (cudaMalloc((void **)&t, need) != cudaSuccess) {
+                        cudaGetLastError();
+                        t = nullptr;
+                    }
+                }
+                if (t) {  // published only once the unpack and the event behind it are enqueued
+                    cudaError_t e = db->tiles_ready ? cudaSuccess : cudaEventCreateWithFlags(&db->tiles_ready, cudaEventDisableTiming);
+                    if (e == cudaSuccess) e = launch_knn2_unpack_tiles(st, db->rows_dev, db->rows, t);
+                    if (e == cudaSuccess) e = cudaEventRecord(db->tiles_ready, st);
+                    if (e != cudaSuccess) {
+                        cudaFree(t);
+                        set_error("knn2 tile build: %s", cudaGetErrorString(e));
+                        return SFE_ERR_CUDA;
+                    }
+                    db->tiles_dev = t;
                     m->launches++;
-                } else {
-                    cudaGetLastError();
-                    db->tiles_dev = nullptr;
                 }
             }
+            if (db->tiles_dev) {
+                SFE_CUDA(cudaStreamWaitEvent(st, db->tiles_ready, 0));  // the unpack may run on another matcher's stream
+                tiles = db->tiles_dev;
+            }
         }
-        SFE_CUDA(launch_knn2_tc(st, m->sm_count, db->rows_dev, db->tiles_dev, db->rows, db->idx_base, (int)chunk_rows, chunks, q_dev, q,
+        SFE_CUDA(launch_knn2_tc(st, m->sm_count, db->rows_dev, tiles, db->rows, db->idx_base, (int)chunk_rows, chunks, q_dev, q,
                                 m->d_part.p));
         if (push)
             knn2_merge_push_kernel<<<div_up(q, 4), 128, 0, st>>>(*push, m->d_part.p, chunks, q);
@@ -2012,6 +2034,7 @@ int sfe_db_destroy(sfe_db *db) {
     SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
     cudaFree(db->rows_dev);
     if (db->tiles_dev) cudaFree(db->tiles_dev);
+    if (db->tiles_ready) cudaEventDestroy(db->tiles_ready);
     delete db;
     return SFE_OK;
 }
