@@ -95,6 +95,7 @@ typedef struct sfe_db sfe_db;
 typedef struct sfe_event sfe_event;
 typedef struct sfe_frame sfe_frame;
 typedef struct sfe_vocab sfe_vocab;
+typedef struct sfe_bowdb sfe_bowdb;
 typedef struct sfe_comm sfe_comm;
 
 /* ---- general -------------------------------------------------------------------------- */
@@ -343,6 +344,35 @@ int sfe_vocab_transform_dev(sfe_matcher *m, const sfe_vocab *v, const uint8_t *d
  * NULL to query the size).  The FeatureVector is node_id -> the feature indices with weight > 0, in feature order. */
 int sfe_bow_assemble(const int32_t *word_id, const double *weight, int n, int weighting, int norm,
                      int32_t *ids, double *values, int cap, int *n_out);
+
+/* ---- BoW database (DBoW2 TemplatedDatabase with L1 scoring: queryL1, L1Scoring::score in GeneralScoring.cpp) ----------
+ * Keyframe BowVectors kept on the device as a forward file (entry offsets, word ids, values), scored against query
+ * BowVectors exactly as DBoW2 does, bit for bit.  Only L1 scoring exists (ORBvoc.txt is "10 6 0 0").
+ * Vectors travel in CSR form: vector i = ids / values [offsets[i], offsets[i+1]); ids must lie in [0, n_words) and ascend
+ * strictly within a vector (a BowVector is a std::map), values must be finite; an empty vector is legal.  Anything else is
+ * SFE_ERR_BAD_ARG and leaves the database unchanged.
+ * Entry ids are 0, 1, 2, ... in add order, as Database::add returns them.
+ * Threads: one database may be used by several matchers of its device, from several threads.  add and query take the
+ * database's lock; a query sees exactly the entries added before it was called.  add is synchronous: when it returns its
+ * vectors are on the device, and before a growing add frees the buffers it outgrew it waits for the queries already
+ * enqueued on any stream. */
+#define SFE_BOWDB_MAX_RESULTS 1024
+int sfe_bowdb_create(sfe_matcher *m, int n_words, sfe_bowdb **out);
+int sfe_bowdb_destroy(sfe_bowdb *db);
+int sfe_bowdb_size(const sfe_bowdb *db, int *entries);
+/* appends `count` vectors; *first_entry (optional) = the id of the first.  Storage grows by doubling. */
+int sfe_bowdb_add(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets /* count + 1 */, const int32_t *ids,
+                  const double *values, int count, int32_t *first_entry);
+/* q queries.  For query i: entry[i*max_results + j], score[i*max_results + j] for j < n_results[i] = the entries that share
+ * at least one word with it and satisfy (e < max_id || max_id == -1), ordered by DBoW2's raw L1 sum with equal sums in
+ * ascending entry id, cut to max_results, score = -sum / 2.0 (Database::query's QueryResults); the rest of the row is
+ * -1 / 0.0.  1 <= max_results <= SFE_BOWDB_MAX_RESULTS (above: SFE_ERR_UNSUPPORTED).  dense (optional, q x dense_entries):
+ * dense[i*dense_entries + e] = L1Scoring::score(query i, entry e) for the entries e < dense_entries whatever max_id, -0.0
+ * where no word is shared -- the similarity matrix.  dense_entries may not exceed the entry count (SFE_ERR_BAD_ARG): a
+ * caller that shares the database with an adding thread passes the count it last observed, as it does for max_id. */
+int sfe_bowdb_query(sfe_matcher *m, const sfe_bowdb *db, const int64_t *offsets /* q + 1 */, const int32_t *ids,
+                    const double *values, int q, int max_id, int max_results, int32_t *entry, double *score,
+                    int32_t *n_results, double *dense, int dense_entries);
 
 /* Sharded ProjectionMatch (map points partitioned over GPUs, frame replicated): each shard emits per keypoint
  * the key (dist << 32 | ~global map-point index) of its best accepted query -- the minimum over shards is the

@@ -315,6 +315,7 @@ public:
         sfe_vocab_destroy(voc_);
         voc_ = nullptr;
         L_ = L;
+        scoring_ = scoring;
         weighting_ = weighting;
         norm_ = scoring == 5 ? 0 : (scoring == 1 ? 2 : 1);  // ScoringObject.h:74-89: DOT_PRODUCT none, L2_NORM L2, the rest L1
         return sfe_vocab_create(thread_matcher(), (int)parent.size(), parent.data(), is_leaf.data(), desc.data(), weight.data(), L,
@@ -322,6 +323,13 @@ public:
     }
 
     bool empty() const { return voc_ == nullptr; }
+    int getScoringType() const { return scoring_; }
+    // number of words (TemplatedVocabulary::size)
+    unsigned int size() const {
+        int n = 0;
+        if (voc_) check(sfe_vocab_words(voc_, &n), "sfe_vocab_words");
+        return (unsigned int)n;
+    }
 
     // void transform(const std::vector<TDescriptor>& features, BowVector &v, FeatureVector &fv, int levelsup) const
     template <class BowVectorT, class FeatureVectorT>
@@ -345,7 +353,77 @@ public:
 
 private:
     sfe_vocab *voc_ = nullptr;
-    int k_ = 0, L_ = 0, weighting_ = 0, norm_ = 1;
+    int k_ = 0, L_ = 0, scoring_ = 0, weighting_ = 0, norm_ = 1;
+};
+
+// DBoW2::TemplatedDatabase stand-in for the loop-candidate query (thirdparty/DBoW2/DBoW2/TemplatedDatabase.h: add, query
+// with L1 scoring = queryL1, size): the keyframe BowVectors stay on the device and every query is scored there, bit for bit.
+// Equal scores come back in ascending entry id.  BowVectorT = any std::map<unsigned, double> (DBoW2::BowVector);
+// QueryResultsT = a vector of a type constructible from (EntryId, double score) (DBoW2::QueryResults of DBoW2::Result).
+// Only L1 scoring exists (ORBvoc.txt is "10 6 0 0"): a vocabulary with another scoring type is rejected.  One Database may
+// be used from several threads (each call uses its thread's matcher handle).  There is no direct index (FeatureVector).
+class Database {
+public:
+    typedef unsigned int EntryId;
+
+    explicit Database(const Vocabulary &voc) {
+        if (voc.empty()) throw std::invalid_argument("sfe_adapter::Database: empty vocabulary");
+        if (voc.getScoringType() != 0)
+            throw std::runtime_error(std::string("sfe_adapter::Database: ") + sfe_status_string(SFE_ERR_UNSUPPORTED) +
+                                     " (only L1_NORM scoring is implemented)");
+        check(sfe_bowdb_create(thread_matcher(), (int)voc.size(), &db_), "sfe_bowdb_create");
+    }
+    ~Database() { sfe_bowdb_destroy(db_); }
+    Database(const Database &) = delete;
+    Database &operator=(const Database &) = delete;
+
+    template <class BowVectorT>
+    EntryId add(const BowVectorT &v) {
+        std::vector<int32_t> ids;
+        std::vector<double> vals;
+        flatten(v, ids, vals);
+        const int64_t off[2] = {0, (int64_t)ids.size()};
+        int32_t first = 0;
+        check(sfe_bowdb_add(thread_matcher(), db_, off, ids.data(), vals.data(), 1, &first), "sfe_bowdb_add");
+        return (EntryId)first;
+    }
+
+    // void query(const BowVector &vec, QueryResults &ret, int max_results = 1, int max_id = -1) const
+    // 1 <= max_results <= SFE_BOWDB_MAX_RESULTS (DBoW2's "max_results <= 0: every entry" is not offered).
+    template <class BowVectorT, class QueryResultsT>
+    void query(const BowVectorT &vec, QueryResultsT &ret, int max_results = 1, int max_id = -1) const {
+        ret.clear();
+        std::vector<int32_t> ids;
+        std::vector<double> vals;
+        flatten(vec, ids, vals);
+        const int64_t off[2] = {0, (int64_t)ids.size()};
+        const int k = max_results;
+        std::vector<int32_t> ent(k > 0 ? k : 1);
+        std::vector<double> sc(k > 0 ? k : 1);
+        int32_t n = 0;
+        check(sfe_bowdb_query(thread_matcher(), db_, off, ids.data(), vals.data(), 1, max_id, k, ent.data(), sc.data(), &n, nullptr, 0),
+              "sfe_bowdb_query");
+        ret.reserve(n);
+        for (int i = 0; i < n; i++) ret.push_back(typename QueryResultsT::value_type((EntryId)ent[i], sc[i]));
+    }
+
+    unsigned int size() const {
+        int n = 0;
+        check(sfe_bowdb_size(db_, &n), "sfe_bowdb_size");
+        return (unsigned int)n;
+    }
+
+private:
+    template <class BowVectorT>
+    static void flatten(const BowVectorT &v, std::vector<int32_t> &ids, std::vector<double> &vals) {
+        ids.reserve(v.size());
+        vals.reserve(v.size());
+        for (const auto &kv : v) {
+            ids.push_back((int32_t)kv.first);
+            vals.push_back((double)kv.second);
+        }
+    }
+    sfe_bowdb *db_ = nullptr;
 };
 
 }  // namespace sfe_adapter

@@ -168,6 +168,11 @@ SIGNATURES = {
     "sfe_vocab_transform": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "sfe_vocab_transform_dev": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "sfe_bow_assemble": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, C.POINTER(_i)]),
+    "sfe_bowdb_create": (_i, [_vp, _i, _pp]),
+    "sfe_bowdb_destroy": (_i, [_vp]),
+    "sfe_bowdb_size": (_i, [_vp, C.POINTER(_i)]),
+    "sfe_bowdb_add": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "sfe_bowdb_query": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _i]),
     "sfe_db_create": (_i, [_vp, _vp, _i64, _i64, _pp]),
     "sfe_db_destroy": (_i, [_vp]),
     "sfe_knn2": (_i, [_vp, _vp, _vp, _i, _vp]),
@@ -842,6 +847,77 @@ def bow_assemble(word_id, weight, weighting=0, norm=1):
     ids, vals = np.zeros(len(word_id), np.int32), np.zeros(len(word_id), np.float64)
     _check(lib().sfe_bow_assemble(_p(word_id), _p(weight), len(word_id), weighting, norm, _p(ids), _p(vals), len(ids), C.byref(n)))
     return ids[:n.value].copy(), vals[:n.value].copy()
+
+
+BOWDB_MAX_RESULTS = 1024  # SFE_BOWDB_MAX_RESULTS
+
+
+def bow_csr(vectors):
+    """BowVectors given as (ids, values) pairs -> (offsets int64[n + 1], ids int32, values float64), the CSR form the
+    BoW database entry points take."""
+    vs = [(np.ascontiguousarray(i, np.int32).reshape(-1), np.ascontiguousarray(v, np.float64).reshape(-1)) for i, v in vectors]
+    for i, v in vs:
+        if len(i) != len(v):
+            raise SfeError(SFE_ERR_BAD_ARG, "a BowVector needs one value per word id")
+    off = np.zeros(len(vs) + 1, np.int64)
+    np.cumsum([len(i) for i, _ in vs], out=off[1:])
+    ids = np.concatenate([i for i, _ in vs] + [np.zeros(0, np.int32)])
+    vals = np.concatenate([v for _, v in vs] + [np.zeros(0, np.float64)])
+    return off, ids, vals
+
+
+class BowDatabase:
+    """DBoW2's keyframe database (TemplatedDatabase) with L1 scoring, resident on the device: add() BowVectors -- the
+    (ids, values) that Vocabulary.transform returns -- and query them as Database::query does, bit for bit.  Entry ids are
+    0, 1, 2, ... in add order.  Several matchers of the device may share one database from several threads."""
+
+    def __init__(self, matcher: "Matcher", n_words):
+        self.m = matcher
+        h = C.c_void_p()
+        _check(lib().sfe_bowdb_create(matcher.h, int(n_words), C.byref(h)))
+        self.h, self.n_words = h, int(n_words)
+
+    def close(self):
+        if getattr(self, "h", None):
+            lib().sfe_bowdb_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __len__(self):
+        n = C.c_int()
+        _check(lib().sfe_bowdb_size(self.h, C.byref(n)))
+        return n.value
+
+    def add(self, vectors, matcher=None) -> int:
+        """Appends BowVectors (a list of (ids, values)) -> the entry id of the first."""
+        off, ids, vals = bow_csr(vectors)
+        first = C.c_int32()
+        _check(lib().sfe_bowdb_add((matcher or self.m).h, self.h, _p(off), _p(ids), _p(vals), len(off) - 1, C.byref(first)))
+        return first.value
+
+    def query(self, vectors, max_results, max_id=-1, dense=False, dense_entries=None, matcher=None):
+        """Database::query(v, ret, max_results, max_id) for every vector -> a list of (entry ids, scores) in DBoW2's order
+        (equal scores by ascending entry id).  dense=True also returns the q x dense_entries matrix of
+        L1Scoring::score(query, entry) for the first dense_entries entries (default: all of them)."""
+        off, ids, vals = bow_csr(vectors)
+        q = len(off) - 1
+        k = int(max_results)
+        ent = np.full((q, max(k, 1)), -1, np.int32)
+        sc = np.zeros((q, max(k, 1)), np.float64)
+        n = np.zeros(q, np.int32)
+        d, de = None, 0
+        if dense:
+            de = len(self) if dense_entries is None else int(dense_entries)
+            d = np.zeros((q, max(de, 0)), np.float64)
+        _check(lib().sfe_bowdb_query((matcher or self.m).h, self.h, _p(off), _p(ids), _p(vals), q, int(max_id), k, _p(ent), _p(sc),
+                                     _p(n), _p(d), de))
+        res = [(ent[i, :n[i]].copy(), sc[i, :n[i]].copy()) for i in range(q)]
+        return (res, d) if dense else res
 
 
 class DescriptorDB:

@@ -1224,6 +1224,10 @@ struct sfe_matcher {
     DevBuf<uint16_t> d_proj_bins;  // sorted ProjectionMatch: bin per map point,
     DevBuf<int> d_proj_hist;       // per-chunk bin histograms + bin totals,
     DevBuf<uint32_t> d_proj_perm;  // map points in bin order
+    DevBuf<int64_t> d_bow_off;     // BoW database queries: CSR of the query batch,
+    DevBuf<int32_t> d_bow_ids, d_bow_e, d_bow_n;
+    DevBuf<double> d_bow_val, d_bow_raw, d_bow_dense, d_bow_s;  // raw L1 sums, dense scores, results
+    DevBuf<uint8_t> d_bow_hit;     // 1 where a query and an entry share a word
 };
 
 struct sfe_db {
@@ -1427,6 +1431,28 @@ static int knn_partial(sfe_matcher *m, const sfe_db *db, const uint8_t *q_dev, i
     return SFE_OK;
 }
 
+namespace sfe {
+cudaError_t launch_bow_score(cudaStream_t st, const int64_t *q_off, const int32_t *q_ids, const double *q_val, int q, int max_nq,
+                             const int64_t *d_off, const int32_t *d_ids, const double *d_val, int n_entries, long long stride,
+                             double *raw, uint8_t *hit, double *dense);
+cudaError_t launch_bow_topk(cudaStream_t st, const double *raw, const uint8_t *hit, long long stride, int q, int n, int k,
+                            int32_t *out_e, double *out_s, int32_t *out_n);
+}
+
+struct sfe_bowdb {
+    int device = 0, n_words = 0;
+    int size = 0;                        // entries
+    int64_t nnz = 0;                     // words over all entries
+    int64_t cap_entries = 0, cap_nnz = 0;
+    int64_t *off = nullptr;              // forward file: entry e = ids / val [off[e], off[e+1])
+    int32_t *ids = nullptr;
+    double *val = nullptr;
+    mutable std::mutex mu;               // guards everything above and `readers`
+    // one event per stream that has queried the database, recorded behind that query's kernels: an add that outgrows the
+    // buffers waits for all of them before it frees the old ones
+    mutable std::vector<std::pair<cudaStream_t, cudaEvent_t>> readers;
+};
+
 extern "C" {
 
 int sfe_matcher_create(int device, sfe_matcher **out) {
@@ -1462,6 +1488,8 @@ int sfe_matcher_destroy(sfe_matcher *m) {
     m->d_n.release(); m->d_idx.release(); m->d_dist.release(); m->d_xw.release(); m->d_grid.release();
     m->d_best.release(); m->d_part.release(); m->d_keys.release(); m->d_quad.release();
     m->d_proj_bins.release(); m->d_proj_hist.release(); m->d_proj_perm.release();
+    m->d_bow_off.release(); m->d_bow_ids.release(); m->d_bow_e.release(); m->d_bow_n.release(); m->d_bow_val.release();
+    m->d_bow_raw.release(); m->d_bow_dense.release(); m->d_bow_s.release(); m->d_bow_hit.release();
     cudaStreamDestroy(m->stream);
     delete m;
     return SFE_OK;
@@ -2003,6 +2031,206 @@ int sfe_bow_assemble(const int32_t *word_id, const double *weight, int n, int we
     *n_out = (int)v.size();
     SFE_REQUIRE((int)v.size() <= cap || (!ids && !values), SFE_ERR_CAPACITY, "BowVector larger than the caller's capacity");
     for (size_t i = 0; i < v.size() && ids && values; i++) { ids[i] = v[i].first; values[i] = v[i].second; }
+    return SFE_OK;
+}
+
+// ---- BoW database (DBoW2 TemplatedDatabase with L1 scoring) -----------------------------------------------------------
+// Vectors arrive from outside the program: CSR offsets from 0, non-decreasing; ids in [0, n_words) and strictly ascending
+// within a vector (a BowVector is a std::map); finite values.
+static int bow_check_vectors(const int64_t *off, const int32_t *ids, const double *val, int count, int n_words) {
+    SFE_REQUIRE(off, SFE_ERR_BAD_ARG, "null offsets");
+    SFE_REQUIRE(off[0] == 0, SFE_ERR_BAD_ARG, "offsets[0] must be 0");
+    for (int i = 0; i < count; i++) SFE_REQUIRE(off[i + 1] >= off[i], SFE_ERR_BAD_ARG, "offsets must not decrease");
+    SFE_REQUIRE(off[count] == 0 || (ids && val), SFE_ERR_BAD_ARG, "null ids / values");
+    for (int i = 0; i < count; i++) {
+        for (int64_t j = off[i]; j < off[i + 1]; j++) {
+            SFE_REQUIRE(ids[j] >= 0 && ids[j] < n_words, SFE_ERR_BAD_ARG, "word id outside [0, n_words)");
+            SFE_REQUIRE(j == off[i] || ids[j] > ids[j - 1], SFE_ERR_BAD_ARG, "word ids must ascend strictly within a vector");
+            SFE_REQUIRE(std::isfinite(val[j]), SFE_ERR_BAD_ARG, "values must be finite");
+        }
+    }
+    return SFE_OK;
+}
+
+int sfe_bowdb_create(sfe_matcher *m, int n_words, sfe_bowdb **out) {
+    SFE_REQUIRE(m && out && n_words >= 1, SFE_ERR_BAD_ARG, "bad argument");
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    sfe_bowdb *db = new sfe_bowdb();
+    db->device = m->device;
+    db->n_words = n_words;
+    db->cap_entries = 64;
+    cudaError_t e = cudaMalloc((void **)&db->off, sizeof(int64_t) * (db->cap_entries + 1));
+    if (e == cudaSuccess) e = cudaMemset(db->off, 0, sizeof(int64_t));
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) {
+        set_error("BoW database: %s", cudaGetErrorString(e));
+        if (db->off) cudaFree(db->off);
+        delete db;
+        return SFE_ERR_CUDA;
+    }
+    *out = db;
+    return SFE_OK;
+}
+
+int sfe_bowdb_destroy(sfe_bowdb *db) {
+    if (!db) return SFE_OK;
+    DeviceGuard g(db->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    for (auto &r : db->readers) {
+        cudaEventSynchronize(r.second);
+        cudaEventDestroy(r.second);
+    }
+    cudaFree(db->off);
+    if (db->ids) cudaFree(db->ids);
+    if (db->val) cudaFree(db->val);
+    delete db;
+    return SFE_OK;
+}
+
+int sfe_bowdb_size(const sfe_bowdb *db, int *entries) {
+    SFE_REQUIRE(db && entries, SFE_ERR_BAD_ARG, "null argument");
+    std::lock_guard<std::mutex> lock(db->mu);
+    *entries = db->size;
+    return SFE_OK;
+}
+
+int sfe_bowdb_add(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets, const int32_t *ids, const double *values, int count,
+                  int32_t *first_entry) {
+    SFE_REQUIRE(m && db && count >= 0, SFE_ERR_BAD_ARG, "bad argument");
+    SFE_REQUIRE(db->device == m->device, SFE_ERR_BAD_ARG, "database lives on another device");
+    int rc = bow_check_vectors(offsets, ids, values, count, db->n_words);
+    if (rc != SFE_OK) return rc;
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    std::lock_guard<std::mutex> lock(db->mu);
+    SFE_REQUIRE((int64_t)db->size + count < INT32_MAX, SFE_ERR_UNSUPPORTED, "entry ids must fit int32");
+    const int32_t first = db->size;
+    if (count > 0) {
+        cudaStream_t st = m->stream;
+        const int64_t add_nnz = offsets[count];
+        const int64_t need_e = (int64_t)db->size + count, need_nnz = db->nnz + add_nnz;
+        int64_t *off = db->off;
+        int32_t *wid = db->ids;
+        double *val = db->val;
+        int64_t cap_e = db->cap_entries, cap_n = db->cap_nnz;
+        if (need_e > cap_e || need_nnz > cap_n) {
+            // capacity doubling: an add costs amortised O(its own size); the old buffers may still be read by queries
+            // enqueued on other streams, so they are freed only once those have run
+            for (auto &r : db->readers) SFE_CUDA(cudaEventSynchronize(r.second));
+            if (need_e > cap_e) cap_e = std::max(need_e, 2 * cap_e);
+            if (need_nnz > cap_n) cap_n = std::max(need_nnz, 2 * cap_n);
+            cudaError_t e = cudaSuccess;
+            if (cap_e != db->cap_entries) e = cudaMalloc((void **)&off, sizeof(int64_t) * (cap_e + 1));
+            if (e == cudaSuccess && cap_n != db->cap_nnz) {
+                wid = nullptr;
+                val = nullptr;
+                e = cudaMalloc((void **)&wid, sizeof(int32_t) * cap_n);
+                if (e == cudaSuccess) e = cudaMalloc((void **)&val, sizeof(double) * cap_n);
+            }
+            if (e == cudaSuccess && off != db->off)
+                e = cudaMemcpyAsync(off, db->off, sizeof(int64_t) * (db->size + 1), cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess && wid != db->ids && db->nnz > 0) {
+                e = cudaMemcpyAsync(wid, db->ids, sizeof(int32_t) * db->nnz, cudaMemcpyDeviceToDevice, st);
+                if (e == cudaSuccess) e = cudaMemcpyAsync(val, db->val, sizeof(double) * db->nnz, cudaMemcpyDeviceToDevice, st);
+            }
+            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+            if (e != cudaSuccess) {  // the database keeps its old buffers and contents
+                if (off != db->off) cudaFree(off);
+                if (wid != db->ids && wid) cudaFree(wid);
+                if (val != db->val && val) cudaFree(val);
+                set_error("BoW database growth: %s", cudaGetErrorString(e));
+                return SFE_ERR_CUDA;
+            }
+            if (off != db->off) cudaFree(db->off);
+            if (wid != db->ids && db->ids) cudaFree(db->ids);
+            if (val != db->val && db->val) cudaFree(db->val);
+            db->off = off; db->ids = wid; db->val = val;
+            db->cap_entries = cap_e; db->cap_nnz = cap_n;
+        }
+        std::vector<int64_t> o(count);  // the new entries' end offsets in the database's forward file
+        for (int i = 0; i < count; i++) o[i] = db->nnz + offsets[i + 1];
+        SFE_CUDA(cudaMemcpyAsync(db->off + db->size + 1, o.data(), sizeof(int64_t) * count, cudaMemcpyHostToDevice, st));
+        if (add_nnz > 0) {
+            SFE_CUDA(cudaMemcpyAsync(db->ids + db->nnz, ids, sizeof(int32_t) * add_nnz, cudaMemcpyHostToDevice, st));
+            SFE_CUDA(cudaMemcpyAsync(db->val + db->nnz, values, sizeof(double) * add_nnz, cudaMemcpyHostToDevice, st));
+        }
+        SFE_CUDA(cudaStreamSynchronize(st));  // synchronous: every stream's later query sees the new entries
+        db->size += count;
+        db->nnz += add_nnz;
+    }
+    if (first_entry) *first_entry = first;
+    return SFE_OK;
+}
+
+int sfe_bowdb_query(sfe_matcher *m, const sfe_bowdb *db, const int64_t *offsets, const int32_t *ids, const double *values, int q,
+                    int max_id, int max_results, int32_t *entry, double *score, int32_t *n_results, double *dense,
+                    int dense_entries) {
+    SFE_REQUIRE(m && db && q >= 0, SFE_ERR_BAD_ARG, "bad argument");
+    SFE_REQUIRE(db->device == m->device, SFE_ERR_BAD_ARG, "database lives on another device");
+    SFE_REQUIRE(max_results >= 1, SFE_ERR_BAD_ARG, "max_results must be >= 1 (the score against every entry is `dense`)");
+    SFE_REQUIRE(max_results <= SFE_BOWDB_MAX_RESULTS, SFE_ERR_UNSUPPORTED, "max_results above SFE_BOWDB_MAX_RESULTS");
+    SFE_REQUIRE(!dense || dense_entries >= 0, SFE_ERR_BAD_ARG, "negative dense_entries");
+    if (q == 0) return SFE_OK;
+    SFE_REQUIRE(entry && score && n_results, SFE_ERR_BAD_ARG, "null argument");
+    int rc = bow_check_vectors(offsets, ids, values, q, db->n_words);
+    if (rc != SFE_OK) return rc;
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    cudaStream_t st = m->stream;
+    const int64_t qnnz = offsets[q];
+    int max_nq = 0;
+    for (int i = 0; i < q; i++) max_nq = std::max(max_nq, (int)(offsets[i + 1] - offsets[i]));
+    SFE_CUDA(m->d_bow_off.ensure(q + 1));
+    SFE_CUDA(m->d_bow_ids.ensure(std::max<int64_t>(qnnz, 1)));
+    SFE_CUDA(m->d_bow_val.ensure(std::max<int64_t>(qnnz, 1)));
+    SFE_CUDA(m->d_bow_e.ensure((size_t)q * max_results));
+    SFE_CUDA(m->d_bow_s.ensure((size_t)q * max_results));
+    SFE_CUDA(m->d_bow_n.ensure(q));
+    SFE_CUDA(cudaMemcpyAsync(m->d_bow_off.p, offsets, sizeof(int64_t) * (q + 1), cudaMemcpyHostToDevice, st));
+    if (qnnz > 0) {
+        SFE_CUDA(cudaMemcpyAsync(m->d_bow_ids.p, ids, sizeof(int32_t) * qnnz, cudaMemcpyHostToDevice, st));
+        SFE_CUDA(cudaMemcpyAsync(m->d_bow_val.p, values, sizeof(double) * qnnz, cudaMemcpyHostToDevice, st));
+    }
+    {
+        std::lock_guard<std::mutex> lock(db->mu);  // the entry count and the buffers this query reads
+        const int size = db->size;
+        SFE_REQUIRE(!dense || dense_entries <= size, SFE_ERR_BAD_ARG, "dense_entries exceeds the database's entry count");
+        const int n_eff = max_id == -1 ? size : (max_id < 0 ? 0 : std::min(max_id, size));  // (int)e < max_id || max_id == -1
+        const int n_score = std::max(n_eff, dense ? dense_entries : 0);
+        // queries in batches whose raw sums (+ hit flags, + dense scores) stay within 256 MB of scratch
+        const size_t per_query = (size_t)std::max(n_score, 1) * (9 + (dense ? 8 : 0));
+        const int qb = (int)std::max<size_t>(1, std::min<size_t>(std::min(q, 65535), ((size_t)256 << 20) / per_query));  // grid.y
+        SFE_CUDA(m->d_bow_raw.ensure((size_t)qb * std::max(n_score, 1)));
+        SFE_CUDA(m->d_bow_hit.ensure((size_t)qb * std::max(n_score, 1)));
+        if (dense) SFE_CUDA(m->d_bow_dense.ensure((size_t)qb * std::max(n_score, 1)));
+        for (int i0 = 0; i0 < q; i0 += qb) {
+            const int nb = std::min(qb, q - i0);
+            SFE_CUDA(launch_bow_score(st, m->d_bow_off.p + i0, m->d_bow_ids.p, m->d_bow_val.p, nb, max_nq, db->off, db->ids, db->val,
+                                      n_score, n_score, m->d_bow_raw.p, m->d_bow_hit.p, dense ? m->d_bow_dense.p : nullptr));
+            SFE_CUDA(launch_bow_topk(st, m->d_bow_raw.p, m->d_bow_hit.p, n_score, nb, n_eff, max_results,
+                                     m->d_bow_e.p + (size_t)i0 * max_results, m->d_bow_s.p + (size_t)i0 * max_results,
+                                     m->d_bow_n.p + i0));
+            m->launches += 2;
+            if (dense && dense_entries > 0)
+                SFE_CUDA(cudaMemcpy2DAsync(dense + (size_t)i0 * dense_entries, sizeof(double) * dense_entries, m->d_bow_dense.p,
+                                           sizeof(double) * n_score, sizeof(double) * dense_entries, nb, cudaMemcpyDeviceToHost, st));
+        }
+        cudaEvent_t *ev = nullptr;
+        for (auto &r : db->readers)
+            if (r.first == st) ev = &r.second;
+        if (!ev) {
+            cudaEvent_t e = nullptr;
+            SFE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            db->readers.emplace_back(st, e);
+            ev = &db->readers.back().second;
+        }
+        SFE_CUDA(cudaEventRecord(*ev, st));
+    }
+    SFE_CUDA(cudaMemcpyAsync(entry, m->d_bow_e.p, sizeof(int32_t) * q * max_results, cudaMemcpyDeviceToHost, st));
+    SFE_CUDA(cudaMemcpyAsync(score, m->d_bow_s.p, sizeof(double) * q * max_results, cudaMemcpyDeviceToHost, st));
+    SFE_CUDA(cudaMemcpyAsync(n_results, m->d_bow_n.p, sizeof(int32_t) * q, cudaMemcpyDeviceToHost, st));
+    SFE_CUDA(cudaStreamSynchronize(st));
     return SFE_OK;
 }
 
