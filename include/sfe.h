@@ -344,6 +344,19 @@ int sfe_vocab_transform_dev(sfe_matcher *m, const sfe_vocab *v, const uint8_t *d
  * NULL to query the size).  The FeatureVector is node_id -> the feature indices with weight > 0, in feature order. */
 int sfe_bow_assemble(const int32_t *word_id, const double *weight, int n, int weighting, int norm,
                      int32_t *ids, double *values, int cap, int *n_out);
+/* sfe_bow_assemble for `count` feature sets at once on the device, bit for bit the same vectors.  Input in the
+ * cap-strided layout of the extractor's _dev outputs: set i = rows [i*stride, i*stride + n_dev[i]) of word_id_dev /
+ * weight_dev (e.g. sfe_vocab_transform_dev run over count * stride rows, n_dev = sfe_stereo_frames_dev's n_l); rows past
+ * n_dev[i] are ignored.  Output: compact CSR on the device, the form sfe_bowdb_add_dev / sfe_bowdb_query_dev take --
+ * bow_off_dev[count + 1] (bow_off_dev[0] = 0), set i's BowVector = bow_ids_dev / bow_val_dev [bow_off_dev[i],
+ * bow_off_dev[i+1]), ids ascending.  Size bow_ids_dev / bow_val_dev for count * stride elements, which always suffices.
+ * stride <= SFE_BOW_ASSEMBLE_MAX_STRIDE (above: SFE_ERR_UNSUPPORTED).  Unknown weighting / norm, null pointers, or an
+ * n_dev[i] outside [0, stride] (found on the device; the outputs are then undefined): SFE_ERR_BAD_ARG.  Synchronous: the
+ * call reads back one status word at its end.  Scratch of count * stride ids and values is kept in the matcher. */
+#define SFE_BOW_ASSEMBLE_MAX_STRIDE 16384
+int sfe_bow_assemble_dev(sfe_matcher *m, const int32_t *word_id_dev, const double *weight_dev, const int32_t *n_dev,
+                         int count, int stride, int weighting, int norm, int64_t *bow_off_dev, int32_t *bow_ids_dev,
+                         double *bow_val_dev);
 
 /* ---- BoW database (DBoW2 TemplatedDatabase with L1 scoring: queryL1, L1Scoring::score in GeneralScoring.cpp) ----------
  * Keyframe BowVectors kept on the device as a forward file (entry offsets, word ids, values), scored against query
@@ -373,6 +386,18 @@ int sfe_bowdb_add(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets /* count
 int sfe_bowdb_query(sfe_matcher *m, const sfe_bowdb *db, const int64_t *offsets /* q + 1 */, const int32_t *ids,
                     const double *values, int q, int max_id, int max_results, int32_t *entry, double *score,
                     int32_t *n_results, double *dense, int dense_entries);
+/* add / query with offsets, ids and values in device memory of the matcher's device (e.g. sfe_bow_assemble_dev's
+ * output); query_dev writes entry, score, n_results and the optional dense matrix to device arrays of the same shapes.
+ * Everything else is the host calls' contract: the same rules (checked on the device by one kernel before anything
+ * changes; a broken rule is SFE_ERR_BAD_ARG and leaves the database unchanged), max_id / max_results / dense_entries,
+ * ties, lock and reader events.  Both read the check's result back once and are synchronous: add_dev's vectors are on
+ * the device (copied device to device) and query_dev's results written when they return.  *first_entry is host memory. */
+int sfe_bowdb_add_dev(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets_dev /* count + 1 */, const int32_t *ids_dev,
+                      const double *values_dev, int count, int32_t *first_entry);
+int sfe_bowdb_query_dev(sfe_matcher *m, const sfe_bowdb *db, const int64_t *offsets_dev /* q + 1 */,
+                        const int32_t *ids_dev, const double *values_dev, int q, int max_id, int max_results,
+                        int32_t *entry_dev, double *score_dev, int32_t *n_results_dev, double *dense_dev,
+                        int dense_entries);
 
 /* Sharded ProjectionMatch (map points partitioned over GPUs, frame replicated): each shard emits per keypoint
  * the key (dist << 32 | ~global map-point index) of its best accepted query -- the minimum over shards is the

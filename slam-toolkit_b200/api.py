@@ -168,11 +168,14 @@ SIGNATURES = {
     "sfe_vocab_transform": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "sfe_vocab_transform_dev": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "sfe_bow_assemble": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, C.POINTER(_i)]),
+    "sfe_bow_assemble_dev": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "sfe_bowdb_create": (_i, [_vp, _i, _pp]),
     "sfe_bowdb_destroy": (_i, [_vp]),
     "sfe_bowdb_size": (_i, [_vp, C.POINTER(_i)]),
     "sfe_bowdb_add": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp]),
     "sfe_bowdb_query": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _i]),
+    "sfe_bowdb_add_dev": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "sfe_bowdb_query_dev": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _i]),
     "sfe_db_create": (_i, [_vp, _vp, _i64, _i64, _pp]),
     "sfe_db_destroy": (_i, [_vp]),
     "sfe_knn2": (_i, [_vp, _vp, _vp, _i, _vp]),
@@ -839,6 +842,19 @@ class Vocabulary:
             fv.setdefault(int(nid[i]), []).append(int(i))
         return (ids, vals), dict(sorted(fv.items()))
 
+    def transform_dev(self, desc_ptr, n_ptr, count, stride, levelsup, word_id_ptr, weight_ptr, node_id_ptr, off_ptr, ids_ptr,
+                      val_ptr):
+        """transform's BowVectors for `count` resident descriptor sets, all on the device: set i = rows [i*stride,
+        i*stride + n[i]) of desc_ptr (int32 counts at n_ptr), e.g. stereo_frames_dev's desc_l / n_l with stride = cap.
+        sfe_vocab_transform_dev over count * stride rows into word_id_ptr / weight_ptr / node_id_ptr, then
+        sfe_bow_assemble_dev with this vocabulary's weighting and norm into the CSR off_ptr (int64, count + 1) /
+        ids_ptr (int32) / val_ptr (float64), the last two sized count * stride."""
+        if stride > BOW_ASSEMBLE_MAX_STRIDE:  # the assembly would reject it: do not write the caller's buffers first
+            raise SfeError(SFE_ERR_UNSUPPORTED, f"stride {stride} above SFE_BOW_ASSEMBLE_MAX_STRIDE ({BOW_ASSEMBLE_MAX_STRIDE})")
+        _check(lib().sfe_vocab_transform_dev(self.m.h, self.h, _p(desc_ptr), count * stride, levelsup, _p(word_id_ptr),
+                                             _p(weight_ptr), _p(node_id_ptr)))
+        bow_assemble_dev(self.m, word_id_ptr, weight_ptr, n_ptr, count, stride, off_ptr, ids_ptr, val_ptr, self.weighting, self.norm)
+
 
 def bow_assemble(word_id, weight, weighting=0, norm=1):
     word_id = np.ascontiguousarray(word_id, np.int32)
@@ -847,6 +863,17 @@ def bow_assemble(word_id, weight, weighting=0, norm=1):
     ids, vals = np.zeros(len(word_id), np.int32), np.zeros(len(word_id), np.float64)
     _check(lib().sfe_bow_assemble(_p(word_id), _p(weight), len(word_id), weighting, norm, _p(ids), _p(vals), len(ids), C.byref(n)))
     return ids[:n.value].copy(), vals[:n.value].copy()
+
+
+BOW_ASSEMBLE_MAX_STRIDE = 16384  # SFE_BOW_ASSEMBLE_MAX_STRIDE
+
+
+def bow_assemble_dev(matcher: "Matcher", word_id_ptr, weight_ptr, n_ptr, count, stride, off_ptr, ids_ptr, val_ptr, weighting=0,
+                     norm=1):
+    """bow_assemble for `count` feature sets on the device (sfe_bow_assemble_dev): set i = rows [i*stride, i*stride + n[i])
+    of the int32 word ids / float64 weights -> CSR off_ptr (int64, count + 1) / ids_ptr / val_ptr (count * stride each)."""
+    _check(lib().sfe_bow_assemble_dev(matcher.h, _p(word_id_ptr), _p(weight_ptr), _p(n_ptr), count, stride, weighting, norm,
+                                      _p(off_ptr), _p(ids_ptr), _p(val_ptr)))
 
 
 BOWDB_MAX_RESULTS = 1024  # SFE_BOWDB_MAX_RESULTS
@@ -918,6 +945,22 @@ class BowDatabase:
                                      _p(n), _p(d), de))
         res = [(ent[i, :n[i]].copy(), sc[i, :n[i]].copy()) for i in range(q)]
         return (res, d) if dense else res
+
+    def add_dev(self, off_ptr, ids_ptr, val_ptr, count, matcher=None) -> int:
+        """Appends `count` BowVectors held on the device in CSR form (e.g. bow_assemble_dev's output) -> the entry id of
+        the first."""
+        first = C.c_int32()
+        _check(lib().sfe_bowdb_add_dev((matcher or self.m).h, self.h, _p(off_ptr), _p(ids_ptr), _p(val_ptr), count, C.byref(first)))
+        return first.value
+
+    def query_dev(self, off_ptr, ids_ptr, val_ptr, q, max_results, entry_ptr, score_ptr, n_ptr, max_id=-1, dense_ptr=None,
+                  dense_entries=0, matcher=None):
+        """query for `q` BowVectors held on the device in CSR form; results stay on the device: entry_ptr (int32) and
+        score_ptr (float64) rows of max_results, n_ptr (int32, q) and, when dense_ptr is given, the q x dense_entries
+        float64 score matrix."""
+        _check(lib().sfe_bowdb_query_dev((matcher or self.m).h, self.h, _p(off_ptr), _p(ids_ptr), _p(val_ptr), q, int(max_id),
+                                         int(max_results), _p(entry_ptr), _p(score_ptr), _p(n_ptr), _p(dense_ptr),
+                                         int(dense_entries)))
 
 
 class DescriptorDB:

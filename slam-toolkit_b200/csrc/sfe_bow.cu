@@ -1,9 +1,12 @@
-// BoW database scoring kernels: DBoW2's L1 query (TemplatedDatabase::queryL1, L1Scoring::score), bit for bit.
+// BoW database scoring kernels: DBoW2's L1 query (TemplatedDatabase::queryL1, L1Scoring::score), bit for bit; the
+// validation of vectors that arrive in device memory; BowVector assembly on the device.
 //
 // Every score is a double sum of fabs(q - d) - fabs(q) - fabs(d) over the words a query and an entry share, taken in
 // ascending word order.  The kernels therefore never reduce as a tree: the lanes of a warp find the common words in
 // parallel, and one ordered chain of additions per (query, entry) pair consumes them in word order.
+#include <algorithm>
 #include <cstdint>
+#include <mutex>
 
 #include "sfe_common.cuh"
 
@@ -240,6 +243,255 @@ cudaError_t launch_bow_topk(cudaStream_t st, const double *raw, const uint8_t *h
                             int32_t *out_e, double *out_s, int32_t *out_n) {
     if (q == 0) return cudaSuccess;
     bow_topk_kernel<<<q, kBowTopkThreads, 0, st>>>(raw, hit, stride, n, k, out_e, out_s, out_n);
+    return cudaGetLastError();
+}
+
+// ---- vectors from device memory: validation and rebasing ---------------------------------------------------------------
+
+// chk[0] = nnz (offsets[count]), chk[1] != 0 when a rule is broken, chk[2] = the longest vector.  The rules are the host
+// check's: offsets[0] == 0 and never decreasing, ids in [0, n_words) and strictly ascending within a vector, values finite.
+// One warp per vector; every read stays inside [0, offsets[count]), the extent the CSR itself declares, so inconsistent
+// offsets are reported rather than followed.  Null ids / values skip the content checks (the host rejects them when nnz > 0).
+__global__ void __launch_bounds__(256) bow_check_kernel(const int64_t *__restrict__ off, const int32_t *__restrict__ ids,
+                                                        const double *__restrict__ val, int count, int n_words,
+                                                        unsigned long long *__restrict__ chk) {
+    const int64_t end = off[count];
+    const int lane = threadIdx.x & 31;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
+    if (warp == 0 && lane == 0) {
+        chk[0] = (unsigned long long)end;
+        if (off[0] != 0) atomicOr(&chk[1], 1ull);
+    }
+    for (int i = warp; i < count; i += n_warps) {
+        const int64_t lo = off[i], hi = off[i + 1];
+        bool bad = hi < lo;
+        if (!bad && ids && val) {
+            const int64_t a = lo > 0 ? lo : 0, b = hi < end ? hi : end;
+            for (int64_t j = a + lane; j < b; j += 32) {
+                const int32_t w = ids[j];
+                bad |= w < 0 || w >= n_words || (j > a && w <= ids[j - 1]) || !isfinite(val[j]);
+            }
+        }
+        bad = __any_sync(0xFFFFFFFFu, bad);
+        if (lane == 0) {
+            if (bad) atomicOr(&chk[1], 1ull);
+            else atomicMax(&chk[2], (unsigned long long)(hi - lo));
+        }
+    }
+}
+
+__global__ void bow_rebase_kernel(const int64_t *__restrict__ src, int count, int64_t base, int64_t *__restrict__ dst) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < count) dst[i] = base + src[i + 1];
+}
+
+cudaError_t launch_bow_check(cudaStream_t st, const int64_t *off, const int32_t *ids, const double *val, int count, int n_words,
+                             unsigned long long *chk) {
+    cudaError_t e = cudaMemsetAsync(chk, 0, sizeof(unsigned long long) * 3, st);
+    if (e != cudaSuccess) return e;
+    const int blocks = std::max(1, std::min((count + 7) / 8, 4096));
+    bow_check_kernel<<<blocks, 256, 0, st>>>(off, ids, val, count, n_words, chk);
+    return cudaGetLastError();
+}
+
+// dst[i] = base + src[i + 1], i < count: a batch's end offsets moved into a forward file that already holds `base` words
+cudaError_t launch_bow_rebase(cudaStream_t st, const int64_t *src, int count, int64_t base, int64_t *dst) {
+    if (count == 0) return cudaSuccess;
+    bow_rebase_kernel<<<(count + 255) / 256, 256, 0, st>>>(src, count, base, dst);
+    return cudaGetLastError();
+}
+
+// ---- BowVector assembly (TemplatedVocabulary::transform's BowVector half, BowVector.cpp:34-84) ---------------------------
+//
+// The host sfe_bow_assemble's order of operations, one CTA per feature set: the accepted features (weight > 0, so NaN is
+// skipped) become keys (word id with the sign bit flipped << 32 | feature index), which a bitonic sort puts in ascending
+// signed word order with each word's features in feature order -- the order std::map insertion sees them.  The first key
+// of each run owns the word: TF_IDF / TF (addWeight) add the run's weights serially in that order, IDF / BINARY
+// (addIfNotExist) keep the first.  The norm is one chain of additions in word order, on one warp.
+
+constexpr int kBowAsmThreads = 1024;
+
+__device__ __forceinline__ int32_t bow_asm_word(unsigned long long key) { return (int32_t)((uint32_t)(key >> 32) ^ 0x80000000u); }
+
+// Set i = rows [i*stride, i*stride + n[i]) of word_id / weight.  Its BowVector goes to rows [i*stride, + cnt[i]) of
+// out_ids / out_val, each value still to be divided by div_out[i] when that is > 0.0.  A count outside [0, stride] sets
+// *status and leaves the set empty.  (The division sits in the compaction: its slow path makes this kernel spill.)
+__global__ void __launch_bounds__(kBowAsmThreads) bow_assemble_kernel(const int32_t *__restrict__ word_id,
+                                                                      const double *__restrict__ weight,
+                                                                      const int32_t *__restrict__ n_set, int stride, int weighting,
+                                                                      int norm, int32_t *__restrict__ cnt,
+                                                                      double *__restrict__ div_out, int32_t *out_ids, double *out_val,
+                                                                      unsigned long long *__restrict__ status) {
+    extern __shared__ __align__(16) unsigned char bow_asm_smem[];
+    unsigned long long *key = (unsigned long long *)bow_asm_smem;
+    __shared__ int wsum[kBowAsmThreads / 32];
+    __shared__ double s_norm;
+    const int set = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const int n = n_set[set];
+    if (n < 0 || n > stride) {  // uniform
+        if (t == 0) {
+            atomicOr(status, 1ull);
+            cnt[set] = 0;
+            div_out[set] = 0.0;
+        }
+        return;
+    }
+    const size_t row0 = (size_t)set * stride;
+    word_id += row0;
+    weight += row0;
+    out_ids += row0;
+    out_val += row0;
+    int P = 1;
+    while (P < n) P <<= 1;
+    int c = 0;  // accepted features
+    for (int f0 = 0; f0 < P; f0 += kBowAsmThreads) {
+        const int f = f0 + t;
+        bool ok = false;
+        if (f < P) {
+            ok = f < n && weight[f] > 0.0;
+            key[f] = ok ? ((unsigned long long)((uint32_t)word_id[f] ^ 0x80000000u) << 32) | (unsigned)f : ~0ull;
+        }
+        c += __syncthreads_count(ok);
+    }
+    for (int size = 2; size <= P; size <<= 1) {
+        for (int j = size >> 1; j > 0; j >>= 1) {
+            for (int x = t; x < P / 2; x += kBowAsmThreads) {
+                const int lo = (x / j) * 2 * j + (x & (j - 1)), hi = lo + j;
+                const unsigned long long a = key[lo], b = key[hi];
+                if ((a > b) == ((lo & size) == 0)) {
+                    key[lo] = b;
+                    key[hi] = a;
+                }
+            }
+            __syncthreads();
+        }
+    }
+    const bool accumulate = weighting == 0 || weighting == 1;
+    int u = 0;  // words so far
+    for (int p0 = 0; p0 < c; p0 += kBowAsmThreads) {  // uniform
+        const int p = p0 + t;
+        const bool head = p < c && (p == 0 || (key[p] >> 32) != (key[p - 1] >> 32));
+        const unsigned bal = __ballot_sync(0xFFFFFFFFu, head);
+        if (lane == 0) wsum[warp] = __popc(bal);
+        __syncthreads();
+        int before = 0, total = 0;
+        for (int w = 0; w < kBowAsmThreads / 32; w++) {
+            if (w < warp) before += wsum[w];
+            total += wsum[w];
+        }
+        if (head) {
+            const unsigned long long k0 = key[p];
+            double v = weight[(uint32_t)k0];
+            if (accumulate)
+                for (int q = p + 1; q < c && (key[q] >> 32) == (k0 >> 32); q++) v = __dadd_rn(v, weight[(uint32_t)key[q]]);
+            const int r = u + before + __popc(bal & ((1u << lane) - 1));
+            out_ids[r] = bow_asm_word(k0);
+            out_val[r] = v;
+        }
+        u += total;
+        __syncthreads();  // wsum is rewritten by the next chunk
+    }
+    // every value is then divided (by bow_compact_kernel) by the word count -- TF_IDF / TF without a norm: "unnecessary when
+    // normalizing" -- or by the norm when it is > 0.0; never both
+    double div = accumulate && norm == 0 ? (double)u : 0.0;
+    if (norm != 0) {
+        if (warp == 0) {  // one serial chain in word order: the lanes fetch 32 terms, the additions consume them in lane order
+            double s = 0.0;
+            for (int r0 = 0; r0 < u; r0 += 32) {
+                const int r = r0 + lane;
+                double x = 0.0;
+                if (r < u) {
+                    const double v = out_val[r];
+                    x = norm == 1 ? fabs(v) : __dmul_rn(v, v);
+                }
+                const int m = min(32, u - r0);
+                for (int l = 0; l < m; l++) s = __dadd_rn(s, __shfl_sync(0xFFFFFFFFu, x, l));
+            }
+            if (lane == 0) s_norm = norm == 2 ? __dsqrt_rn(s) : s;
+        }
+        __syncthreads();
+        div = s_norm;
+    }
+    if (t == 0) {
+        cnt[set] = u;
+        div_out[set] = div;
+    }
+}
+
+// off[0] = 0, off[i + 1] = off[i] + cnt[i]: one CTA, a block-wide scan per chunk of kBowAsmThreads sets
+__global__ void __launch_bounds__(kBowAsmThreads) bow_offsets_kernel(const int32_t *__restrict__ cnt, int count,
+                                                                     int64_t *__restrict__ off) {
+    __shared__ long long wsum[kBowAsmThreads / 32];
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    long long base = 0;
+    if (t == 0) off[0] = 0;
+    for (int i0 = 0; i0 < count; i0 += kBowAsmThreads) {
+        const int i = i0 + t;
+        long long v = i < count ? cnt[i] : 0;
+        for (int o = 1; o < 32; o <<= 1) {  // inclusive warp scan
+            const long long y = __shfl_up_sync(0xFFFFFFFFu, v, o);
+            if (lane >= o) v += y;
+        }
+        if (lane == 31) wsum[warp] = v;
+        __syncthreads();
+        long long before = 0, total = 0;
+        for (int w = 0; w < kBowAsmThreads / 32; w++) {
+            if (w < warp) before += wsum[w];
+            total += wsum[w];
+        }
+        if (i < count) off[i + 1] = base + before + v;
+        base += total;
+        __syncthreads();
+    }
+}
+
+// rows [set*stride, + cnt[set]) of the strided vectors -> [off[set], off[set + 1]) of the compact CSR, values divided by
+// div[set] when that is > 0.0
+__global__ void __launch_bounds__(256) bow_compact_kernel(const int32_t *__restrict__ cnt, const double *__restrict__ div,
+                                                          const int64_t *__restrict__ off, int stride,
+                                                          const int32_t *__restrict__ src_ids, const double *__restrict__ src_val,
+                                                          int32_t *__restrict__ dst_ids, double *__restrict__ dst_val) {
+    const int set = blockIdx.x;
+    const int u = cnt[set];
+    const double d = div[set];
+    const size_t s0 = (size_t)set * stride;
+    const int64_t d0 = off[set];
+    for (int r = threadIdx.x; r < u; r += blockDim.x) {
+        const double v = src_val[s0 + r];
+        dst_ids[d0 + r] = src_ids[s0 + r];
+        dst_val[d0 + r] = d > 0.0 ? __ddiv_rn(v, d) : v;
+    }
+}
+
+// count sets of at most stride (<= SFE_BOW_ASSEMBLE_MAX_STRIDE) features -> compact CSR; cnt / div / tmp_ids / tmp_val:
+// scratch of count, count, count * stride, count * stride elements.  *status is set when a set's feature count lies outside [0, stride].
+cudaError_t launch_bow_assemble(cudaStream_t st, const int32_t *word_id, const double *weight, const int32_t *n_set, int count,
+                                int stride, int weighting, int norm, int32_t *cnt, double *div, int32_t *tmp_ids, double *tmp_val,
+                                unsigned long long *status, int64_t *off, int32_t *ids, double *val) {
+    cudaError_t e = cudaMemsetAsync(status, 0, sizeof(unsigned long long), st);
+    if (e != cudaSuccess) return e;
+    if (count == 0) return cudaMemsetAsync(off, 0, sizeof(int64_t), st);
+    // the opt-in limit belongs to the function on the device, shared by every matcher: set once per device, to what the
+    // largest stride needs, so no call ever lowers it under another thread's launch
+    static std::once_flag once[64];
+    static cudaError_t configured[64];
+    int dev = 0;
+    e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    std::call_once(once[dev & 63], [&] {
+        configured[dev & 63] = cudaFuncSetAttribute(bow_assemble_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                    (int)(sizeof(unsigned long long) * SFE_BOW_ASSEMBLE_MAX_STRIDE));
+    });
+    if (configured[dev & 63] != cudaSuccess) return configured[dev & 63];
+    int P = 1;
+    while (P < stride) P <<= 1;
+    const size_t smem = sizeof(unsigned long long) * P;
+    bow_assemble_kernel<<<count, kBowAsmThreads, smem, st>>>(word_id, weight, n_set, stride, weighting, norm, cnt, div, tmp_ids,
+                                                             tmp_val, status);
+    e = cudaGetLastError();  // the scan and the compaction read what the assembly wrote: never enqueue them behind a failure
+    if (e != cudaSuccess) return e;
+    bow_offsets_kernel<<<1, kBowAsmThreads, 0, st>>>(cnt, count, off);
+    bow_compact_kernel<<<count, 256, 0, st>>>(cnt, div, off, stride, tmp_ids, tmp_val, ids, val);
     return cudaGetLastError();
 }
 

@@ -1228,6 +1228,9 @@ struct sfe_matcher {
     DevBuf<int32_t> d_bow_ids, d_bow_e, d_bow_n;
     DevBuf<double> d_bow_val, d_bow_raw, d_bow_dense, d_bow_s;  // raw L1 sums, dense scores, results
     DevBuf<uint8_t> d_bow_hit;     // 1 where a query and an entry share a word
+    DevBuf<unsigned long long> d_bow_chk;  // device vectors: nnz, rule broken, longest vector / assembly status
+    DevBuf<int32_t> d_bowa_cnt, d_bowa_ids;  // BowVector assembly: words per set, vectors at the input's row stride,
+    DevBuf<double> d_bowa_div, d_bowa_val;   // the divisor of each set's values
 };
 
 struct sfe_db {
@@ -1437,6 +1440,12 @@ cudaError_t launch_bow_score(cudaStream_t st, const int64_t *q_off, const int32_
                              double *raw, uint8_t *hit, double *dense);
 cudaError_t launch_bow_topk(cudaStream_t st, const double *raw, const uint8_t *hit, long long stride, int q, int n, int k,
                             int32_t *out_e, double *out_s, int32_t *out_n);
+cudaError_t launch_bow_check(cudaStream_t st, const int64_t *off, const int32_t *ids, const double *val, int count, int n_words,
+                             unsigned long long *chk);
+cudaError_t launch_bow_rebase(cudaStream_t st, const int64_t *src, int count, int64_t base, int64_t *dst);
+cudaError_t launch_bow_assemble(cudaStream_t st, const int32_t *word_id, const double *weight, const int32_t *n_set, int count,
+                                int stride, int weighting, int norm, int32_t *cnt, double *div, int32_t *tmp_ids, double *tmp_val,
+                                unsigned long long *status, int64_t *off, int32_t *ids, double *val);
 }
 
 struct sfe_bowdb {
@@ -1490,6 +1499,7 @@ int sfe_matcher_destroy(sfe_matcher *m) {
     m->d_proj_bins.release(); m->d_proj_hist.release(); m->d_proj_perm.release();
     m->d_bow_off.release(); m->d_bow_ids.release(); m->d_bow_e.release(); m->d_bow_n.release(); m->d_bow_val.release();
     m->d_bow_raw.release(); m->d_bow_dense.release(); m->d_bow_s.release(); m->d_bow_hit.release();
+    m->d_bow_chk.release(); m->d_bowa_cnt.release(); m->d_bowa_div.release(); m->d_bowa_ids.release(); m->d_bowa_val.release();
     cudaStreamDestroy(m->stream);
     delete m;
     return SFE_OK;
@@ -2034,6 +2044,32 @@ int sfe_bow_assemble(const int32_t *word_id, const double *weight, int n, int we
     return SFE_OK;
 }
 
+// The same assembly for `count` feature sets on the device (bow_assemble_kernel, csrc/sfe_bow.cu), bit for bit.
+int sfe_bow_assemble_dev(sfe_matcher *m, const int32_t *word_id_dev, const double *weight_dev, const int32_t *n_dev, int count,
+                         int stride, int weighting, int norm, int64_t *bow_off_dev, int32_t *bow_ids_dev, double *bow_val_dev) {
+    SFE_REQUIRE(m && count >= 0 && stride >= 0 && bow_off_dev, SFE_ERR_BAD_ARG, "bad argument");
+    SFE_REQUIRE(weighting >= 0 && weighting <= 3 && norm >= 0 && norm <= 2, SFE_ERR_BAD_ARG, "unknown weighting / norm");
+    SFE_REQUIRE(count == 0 || (word_id_dev && weight_dev && n_dev && bow_ids_dev && bow_val_dev), SFE_ERR_BAD_ARG, "null argument");
+    SFE_REQUIRE(stride <= SFE_BOW_ASSEMBLE_MAX_STRIDE, SFE_ERR_UNSUPPORTED, "stride above SFE_BOW_ASSEMBLE_MAX_STRIDE");
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    cudaStream_t st = m->stream;
+    const size_t rows = std::max<size_t>((size_t)count * stride, 1);
+    SFE_CUDA(m->d_bow_chk.ensure(3));
+    SFE_CUDA(m->d_bowa_cnt.ensure(std::max(count, 1)));
+    SFE_CUDA(m->d_bowa_div.ensure(std::max(count, 1)));
+    SFE_CUDA(m->d_bowa_ids.ensure(rows));
+    SFE_CUDA(m->d_bowa_val.ensure(rows));
+    SFE_CUDA(launch_bow_assemble(st, word_id_dev, weight_dev, n_dev, count, stride, weighting, norm, m->d_bowa_cnt.p, m->d_bowa_div.p,
+                                 m->d_bowa_ids.p, m->d_bowa_val.p, m->d_bow_chk.p, bow_off_dev, bow_ids_dev, bow_val_dev));
+    m->launches += count > 0 ? 3 : 0;
+    unsigned long long status = 0;
+    SFE_CUDA(cudaMemcpyAsync(&status, m->d_bow_chk.p, sizeof(status), cudaMemcpyDeviceToHost, st));
+    SFE_CUDA(cudaStreamSynchronize(st));
+    SFE_REQUIRE(status == 0, SFE_ERR_BAD_ARG, "a feature count n_dev[i] outside [0, stride]");
+    return SFE_OK;
+}
+
 // ---- BoW database (DBoW2 TemplatedDatabase with L1 scoring) -----------------------------------------------------------
 // Vectors arrive from outside the program: CSR offsets from 0, non-decreasing; ids in [0, n_words) and strictly ascending
 // within a vector (a BowVector is a std::map); finite values.
@@ -2095,6 +2131,66 @@ int sfe_bowdb_size(const sfe_bowdb *db, int *entries) {
     return SFE_OK;
 }
 
+// Room for `count` more entries of `add_nnz` more words; the caller holds db->mu.  Capacity doubling: an add costs amortised
+// O(its own size).  The old buffers may still be read by queries enqueued on other streams, so they are freed only once
+// those have run.  On failure the database keeps its old buffers and contents.
+static int bow_reserve(sfe_bowdb *db, cudaStream_t st, int count, int64_t add_nnz) {
+    const int64_t need_e = (int64_t)db->size + count, need_nnz = db->nnz + add_nnz;
+    int64_t *off = db->off;
+    int32_t *wid = db->ids;
+    double *val = db->val;
+    int64_t cap_e = db->cap_entries, cap_n = db->cap_nnz;
+    if (need_e <= cap_e && need_nnz <= cap_n) return SFE_OK;
+    for (auto &r : db->readers) SFE_CUDA(cudaEventSynchronize(r.second));
+    if (need_e > cap_e) cap_e = std::max(need_e, 2 * cap_e);
+    if (need_nnz > cap_n) cap_n = std::max(need_nnz, 2 * cap_n);
+    cudaError_t e = cudaSuccess;
+    if (cap_e != db->cap_entries) e = cudaMalloc((void **)&off, sizeof(int64_t) * (cap_e + 1));
+    if (e == cudaSuccess && cap_n != db->cap_nnz) {
+        wid = nullptr;
+        val = nullptr;
+        e = cudaMalloc((void **)&wid, sizeof(int32_t) * cap_n);
+        if (e == cudaSuccess) e = cudaMalloc((void **)&val, sizeof(double) * cap_n);
+    }
+    if (e == cudaSuccess && off != db->off)
+        e = cudaMemcpyAsync(off, db->off, sizeof(int64_t) * (db->size + 1), cudaMemcpyDeviceToDevice, st);
+    if (e == cudaSuccess && wid != db->ids && db->nnz > 0) {
+        e = cudaMemcpyAsync(wid, db->ids, sizeof(int32_t) * db->nnz, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(val, db->val, sizeof(double) * db->nnz, cudaMemcpyDeviceToDevice, st);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) {
+        if (off != db->off) cudaFree(off);
+        if (wid != db->ids && wid) cudaFree(wid);
+        if (val != db->val && val) cudaFree(val);
+        set_error("BoW database growth: %s", cudaGetErrorString(e));
+        return SFE_ERR_CUDA;
+    }
+    if (off != db->off) cudaFree(db->off);
+    if (wid != db->ids && db->ids) cudaFree(db->ids);
+    if (val != db->val && db->val) cudaFree(db->val);
+    db->off = off; db->ids = wid; db->val = val;
+    db->cap_entries = cap_e; db->cap_nnz = cap_n;
+    return SFE_OK;
+}
+
+// Vectors in device memory, checked there (bow_check_kernel) with the host check's rules -> their nnz and longest vector.
+static int bow_check_vectors_dev(sfe_matcher *m, const int64_t *off, const int32_t *ids, const double *val, int count, int n_words,
+                                 int64_t *nnz, int *max_len) {
+    SFE_CUDA(m->d_bow_chk.ensure(3));
+    SFE_CUDA(launch_bow_check(m->stream, off, ids, val, count, n_words, m->d_bow_chk.p));
+    m->launches++;
+    unsigned long long chk[3];
+    SFE_CUDA(cudaMemcpyAsync(chk, m->d_bow_chk.p, sizeof(chk), cudaMemcpyDeviceToHost, m->stream));
+    SFE_CUDA(cudaStreamSynchronize(m->stream));
+    SFE_REQUIRE(chk[1] == 0, SFE_ERR_BAD_ARG, "offsets[0] != 0, decreasing offsets, a word id outside [0, n_words) or not "
+                                              "strictly ascending within a vector, or a value that is not finite");
+    *nnz = (int64_t)chk[0];
+    SFE_REQUIRE(*nnz == 0 || (ids && val), SFE_ERR_BAD_ARG, "null ids / values");
+    *max_len = (int)std::min<unsigned long long>(chk[2], INT32_MAX);
+    return SFE_OK;
+}
+
 int sfe_bowdb_add(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets, const int32_t *ids, const double *values, int count,
                   int32_t *first_entry) {
     SFE_REQUIRE(m && db && count >= 0, SFE_ERR_BAD_ARG, "bad argument");
@@ -2109,45 +2205,8 @@ int sfe_bowdb_add(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets, const i
     if (count > 0) {
         cudaStream_t st = m->stream;
         const int64_t add_nnz = offsets[count];
-        const int64_t need_e = (int64_t)db->size + count, need_nnz = db->nnz + add_nnz;
-        int64_t *off = db->off;
-        int32_t *wid = db->ids;
-        double *val = db->val;
-        int64_t cap_e = db->cap_entries, cap_n = db->cap_nnz;
-        if (need_e > cap_e || need_nnz > cap_n) {
-            // capacity doubling: an add costs amortised O(its own size); the old buffers may still be read by queries
-            // enqueued on other streams, so they are freed only once those have run
-            for (auto &r : db->readers) SFE_CUDA(cudaEventSynchronize(r.second));
-            if (need_e > cap_e) cap_e = std::max(need_e, 2 * cap_e);
-            if (need_nnz > cap_n) cap_n = std::max(need_nnz, 2 * cap_n);
-            cudaError_t e = cudaSuccess;
-            if (cap_e != db->cap_entries) e = cudaMalloc((void **)&off, sizeof(int64_t) * (cap_e + 1));
-            if (e == cudaSuccess && cap_n != db->cap_nnz) {
-                wid = nullptr;
-                val = nullptr;
-                e = cudaMalloc((void **)&wid, sizeof(int32_t) * cap_n);
-                if (e == cudaSuccess) e = cudaMalloc((void **)&val, sizeof(double) * cap_n);
-            }
-            if (e == cudaSuccess && off != db->off)
-                e = cudaMemcpyAsync(off, db->off, sizeof(int64_t) * (db->size + 1), cudaMemcpyDeviceToDevice, st);
-            if (e == cudaSuccess && wid != db->ids && db->nnz > 0) {
-                e = cudaMemcpyAsync(wid, db->ids, sizeof(int32_t) * db->nnz, cudaMemcpyDeviceToDevice, st);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(val, db->val, sizeof(double) * db->nnz, cudaMemcpyDeviceToDevice, st);
-            }
-            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-            if (e != cudaSuccess) {  // the database keeps its old buffers and contents
-                if (off != db->off) cudaFree(off);
-                if (wid != db->ids && wid) cudaFree(wid);
-                if (val != db->val && val) cudaFree(val);
-                set_error("BoW database growth: %s", cudaGetErrorString(e));
-                return SFE_ERR_CUDA;
-            }
-            if (off != db->off) cudaFree(db->off);
-            if (wid != db->ids && db->ids) cudaFree(db->ids);
-            if (val != db->val && db->val) cudaFree(db->val);
-            db->off = off; db->ids = wid; db->val = val;
-            db->cap_entries = cap_e; db->cap_nnz = cap_n;
-        }
+        rc = bow_reserve(db, st, count, add_nnz);
+        if (rc != SFE_OK) return rc;
         std::vector<int64_t> o(count);  // the new entries' end offsets in the database's forward file
         for (int i = 0; i < count; i++) o[i] = db->nnz + offsets[i + 1];
         SFE_CUDA(cudaMemcpyAsync(db->off + db->size + 1, o.data(), sizeof(int64_t) * count, cudaMemcpyHostToDevice, st));
@@ -2160,6 +2219,48 @@ int sfe_bowdb_add(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets, const i
         db->nnz += add_nnz;
     }
     if (first_entry) *first_entry = first;
+    return SFE_OK;
+}
+
+// Enqueues the scoring of q query vectors (CSR in device memory, the longest max_nq words) under the database's lock: the
+// top-k rows go to entry / score / n_results (device), the dense rows are copied to `dense` with `dense_kind`, and the
+// stream's reader event is recorded behind them.
+static int bow_query_enqueue(sfe_matcher *m, const sfe_bowdb *db, const int64_t *q_off, const int32_t *q_ids, const double *q_val,
+                             int q, int max_nq, int max_id, int max_results, int32_t *entry, double *score, int32_t *n_results,
+                             double *dense, int dense_entries, cudaMemcpyKind dense_kind) {
+    cudaStream_t st = m->stream;
+    std::lock_guard<std::mutex> lock(db->mu);  // the entry count and the buffers this query reads
+    const int size = db->size;
+    SFE_REQUIRE(!dense || dense_entries <= size, SFE_ERR_BAD_ARG, "dense_entries exceeds the database's entry count");
+    const int n_eff = max_id == -1 ? size : (max_id < 0 ? 0 : std::min(max_id, size));  // (int)e < max_id || max_id == -1
+    const int n_score = std::max(n_eff, dense ? dense_entries : 0);
+    // queries in batches whose raw sums (+ hit flags, + dense scores) stay within 256 MB of scratch
+    const size_t per_query = (size_t)std::max(n_score, 1) * (9 + (dense ? 8 : 0));
+    const int qb = (int)std::max<size_t>(1, std::min<size_t>(std::min(q, 65535), ((size_t)256 << 20) / per_query));  // grid.y
+    SFE_CUDA(m->d_bow_raw.ensure((size_t)qb * std::max(n_score, 1)));
+    SFE_CUDA(m->d_bow_hit.ensure((size_t)qb * std::max(n_score, 1)));
+    if (dense) SFE_CUDA(m->d_bow_dense.ensure((size_t)qb * std::max(n_score, 1)));
+    for (int i0 = 0; i0 < q; i0 += qb) {
+        const int nb = std::min(qb, q - i0);
+        SFE_CUDA(launch_bow_score(st, q_off + i0, q_ids, q_val, nb, max_nq, db->off, db->ids, db->val, n_score, n_score,
+                                  m->d_bow_raw.p, m->d_bow_hit.p, dense ? m->d_bow_dense.p : nullptr));
+        SFE_CUDA(launch_bow_topk(st, m->d_bow_raw.p, m->d_bow_hit.p, n_score, nb, n_eff, max_results, entry + (size_t)i0 * max_results,
+                                 score + (size_t)i0 * max_results, n_results + i0));
+        m->launches += 2;
+        if (dense && dense_entries > 0)
+            SFE_CUDA(cudaMemcpy2DAsync(dense + (size_t)i0 * dense_entries, sizeof(double) * dense_entries, m->d_bow_dense.p,
+                                       sizeof(double) * n_score, sizeof(double) * dense_entries, nb, dense_kind, st));
+    }
+    cudaEvent_t *ev = nullptr;
+    for (auto &r : db->readers)
+        if (r.first == st) ev = &r.second;
+    if (!ev) {
+        cudaEvent_t e = nullptr;
+        SFE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        db->readers.emplace_back(st, e);
+        ev = &db->readers.back().second;
+    }
+    SFE_CUDA(cudaEventRecord(*ev, st));
     return SFE_OK;
 }
 
@@ -2192,45 +2293,69 @@ int sfe_bowdb_query(sfe_matcher *m, const sfe_bowdb *db, const int64_t *offsets,
         SFE_CUDA(cudaMemcpyAsync(m->d_bow_ids.p, ids, sizeof(int32_t) * qnnz, cudaMemcpyHostToDevice, st));
         SFE_CUDA(cudaMemcpyAsync(m->d_bow_val.p, values, sizeof(double) * qnnz, cudaMemcpyHostToDevice, st));
     }
-    {
-        std::lock_guard<std::mutex> lock(db->mu);  // the entry count and the buffers this query reads
-        const int size = db->size;
-        SFE_REQUIRE(!dense || dense_entries <= size, SFE_ERR_BAD_ARG, "dense_entries exceeds the database's entry count");
-        const int n_eff = max_id == -1 ? size : (max_id < 0 ? 0 : std::min(max_id, size));  // (int)e < max_id || max_id == -1
-        const int n_score = std::max(n_eff, dense ? dense_entries : 0);
-        // queries in batches whose raw sums (+ hit flags, + dense scores) stay within 256 MB of scratch
-        const size_t per_query = (size_t)std::max(n_score, 1) * (9 + (dense ? 8 : 0));
-        const int qb = (int)std::max<size_t>(1, std::min<size_t>(std::min(q, 65535), ((size_t)256 << 20) / per_query));  // grid.y
-        SFE_CUDA(m->d_bow_raw.ensure((size_t)qb * std::max(n_score, 1)));
-        SFE_CUDA(m->d_bow_hit.ensure((size_t)qb * std::max(n_score, 1)));
-        if (dense) SFE_CUDA(m->d_bow_dense.ensure((size_t)qb * std::max(n_score, 1)));
-        for (int i0 = 0; i0 < q; i0 += qb) {
-            const int nb = std::min(qb, q - i0);
-            SFE_CUDA(launch_bow_score(st, m->d_bow_off.p + i0, m->d_bow_ids.p, m->d_bow_val.p, nb, max_nq, db->off, db->ids, db->val,
-                                      n_score, n_score, m->d_bow_raw.p, m->d_bow_hit.p, dense ? m->d_bow_dense.p : nullptr));
-            SFE_CUDA(launch_bow_topk(st, m->d_bow_raw.p, m->d_bow_hit.p, n_score, nb, n_eff, max_results,
-                                     m->d_bow_e.p + (size_t)i0 * max_results, m->d_bow_s.p + (size_t)i0 * max_results,
-                                     m->d_bow_n.p + i0));
-            m->launches += 2;
-            if (dense && dense_entries > 0)
-                SFE_CUDA(cudaMemcpy2DAsync(dense + (size_t)i0 * dense_entries, sizeof(double) * dense_entries, m->d_bow_dense.p,
-                                           sizeof(double) * n_score, sizeof(double) * dense_entries, nb, cudaMemcpyDeviceToHost, st));
-        }
-        cudaEvent_t *ev = nullptr;
-        for (auto &r : db->readers)
-            if (r.first == st) ev = &r.second;
-        if (!ev) {
-            cudaEvent_t e = nullptr;
-            SFE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            db->readers.emplace_back(st, e);
-            ev = &db->readers.back().second;
-        }
-        SFE_CUDA(cudaEventRecord(*ev, st));
-    }
+    rc = bow_query_enqueue(m, db, m->d_bow_off.p, m->d_bow_ids.p, m->d_bow_val.p, q, max_nq, max_id, max_results, m->d_bow_e.p,
+                           m->d_bow_s.p, m->d_bow_n.p, dense, dense_entries, cudaMemcpyDeviceToHost);
+    if (rc != SFE_OK) return rc;
     SFE_CUDA(cudaMemcpyAsync(entry, m->d_bow_e.p, sizeof(int32_t) * q * max_results, cudaMemcpyDeviceToHost, st));
     SFE_CUDA(cudaMemcpyAsync(score, m->d_bow_s.p, sizeof(double) * q * max_results, cudaMemcpyDeviceToHost, st));
     SFE_CUDA(cudaMemcpyAsync(n_results, m->d_bow_n.p, sizeof(int32_t) * q, cudaMemcpyDeviceToHost, st));
     SFE_CUDA(cudaStreamSynchronize(st));
+    return SFE_OK;
+}
+
+// add / query with the vectors (and query's results) in device memory: validated there, then the host calls' paths
+int sfe_bowdb_add_dev(sfe_matcher *m, sfe_bowdb *db, const int64_t *offsets_dev, const int32_t *ids_dev, const double *values_dev,
+                      int count, int32_t *first_entry) {
+    SFE_REQUIRE(m && db && count >= 0, SFE_ERR_BAD_ARG, "bad argument");
+    SFE_REQUIRE(db->device == m->device, SFE_ERR_BAD_ARG, "database lives on another device");
+    SFE_REQUIRE(offsets_dev, SFE_ERR_BAD_ARG, "null offsets");
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    int64_t add_nnz = 0;
+    int max_len = 0;
+    int rc = bow_check_vectors_dev(m, offsets_dev, ids_dev, values_dev, count, db->n_words, &add_nnz, &max_len);
+    if (rc != SFE_OK) return rc;
+    std::lock_guard<std::mutex> lock(db->mu);
+    SFE_REQUIRE((int64_t)db->size + count < INT32_MAX, SFE_ERR_UNSUPPORTED, "entry ids must fit int32");
+    const int32_t first = db->size;
+    if (count > 0) {
+        cudaStream_t st = m->stream;
+        rc = bow_reserve(db, st, count, add_nnz);
+        if (rc != SFE_OK) return rc;
+        SFE_CUDA(launch_bow_rebase(st, offsets_dev, count, db->nnz, db->off + db->size + 1));
+        m->launches++;
+        if (add_nnz > 0) {
+            SFE_CUDA(cudaMemcpyAsync(db->ids + db->nnz, ids_dev, sizeof(int32_t) * add_nnz, cudaMemcpyDeviceToDevice, st));
+            SFE_CUDA(cudaMemcpyAsync(db->val + db->nnz, values_dev, sizeof(double) * add_nnz, cudaMemcpyDeviceToDevice, st));
+        }
+        SFE_CUDA(cudaStreamSynchronize(st));  // synchronous: every stream's later query sees the new entries
+        db->size += count;
+        db->nnz += add_nnz;
+    }
+    if (first_entry) *first_entry = first;
+    return SFE_OK;
+}
+
+int sfe_bowdb_query_dev(sfe_matcher *m, const sfe_bowdb *db, const int64_t *offsets_dev, const int32_t *ids_dev,
+                        const double *values_dev, int q, int max_id, int max_results, int32_t *entry_dev, double *score_dev,
+                        int32_t *n_results_dev, double *dense_dev, int dense_entries) {
+    SFE_REQUIRE(m && db && q >= 0, SFE_ERR_BAD_ARG, "bad argument");
+    SFE_REQUIRE(db->device == m->device, SFE_ERR_BAD_ARG, "database lives on another device");
+    SFE_REQUIRE(max_results >= 1, SFE_ERR_BAD_ARG, "max_results must be >= 1 (the score against every entry is `dense`)");
+    SFE_REQUIRE(max_results <= SFE_BOWDB_MAX_RESULTS, SFE_ERR_UNSUPPORTED, "max_results above SFE_BOWDB_MAX_RESULTS");
+    SFE_REQUIRE(!dense_dev || dense_entries >= 0, SFE_ERR_BAD_ARG, "negative dense_entries");
+    if (q == 0) return SFE_OK;
+    SFE_REQUIRE(entry_dev && score_dev && n_results_dev && offsets_dev, SFE_ERR_BAD_ARG, "null argument");
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    int64_t qnnz = 0;
+    int max_nq = 0;
+    int rc = bow_check_vectors_dev(m, offsets_dev, ids_dev, values_dev, q, db->n_words, &qnnz, &max_nq);
+    if (rc != SFE_OK) return rc;
+    rc = bow_query_enqueue(m, db, offsets_dev, ids_dev, values_dev, q, max_nq, max_id, max_results, entry_dev, score_dev,
+                           n_results_dev, dense_dev, dense_entries, cudaMemcpyDeviceToDevice);
+    if (rc != SFE_OK) return rc;
+    SFE_CUDA(cudaStreamSynchronize(m->stream));
     return SFE_OK;
 }
 
