@@ -425,6 +425,30 @@ int sfe_projection_merge_dev(sfe_matcher *m, const uint64_t *keys_dev, int shard
 int sfe_db_create(sfe_matcher *m, const uint8_t *desc_host, int64_t rows, int64_t idx_base,
                   sfe_db **out);
 int sfe_db_destroy(sfe_db *db);
+/* Growing a database in place, e.g. by each keyframe's descriptors.
+ * Indices: appended rows continue the numbering: row r has global index idx_base + r.  An append that would take
+ * idx_base + rows to 2^31 returns SFE_ERR_UNSUPPORTED and leaves the database unchanged.  The library knows nothing of
+ * other shards: a caller that appends to one shard of a row-sharded map keeps the shards' global ranges disjoint itself
+ * (e.g. by appending only to the shard with the highest idx_base).
+ * Arguments: null pointers, rows < 0, count < 0, stride < 1 or a desc_dev that is not 16-byte aligned (every allocation of
+ * the library or torch is) return SFE_ERR_BAD_ARG.  An n_dev[i] outside [0, stride] is found on the device before anything
+ * changes: SFE_ERR_BAD_ARG, the database unchanged.  Appending zero rows succeeds and changes nothing.
+ * Synchronous: when an append returns, its rows (and their tensor-core tiles, where the database keeps them) are on the
+ * device.  append_dev reads one word (the checked total) back.
+ * Threads: several matchers of the device may append to and search one database from several threads.  Appends and every
+ * search (sfe_knn2, sfe_knn2_dev, sfe_knn2_sharded) take the database's lock; a search sees exactly the rows appended
+ * before it was called, also when it is still queued when a later append runs: an append waits for the queued searches
+ * before it frees the buffers it outgrew or rewrites the tile that holds the old last row.
+ * Storage grows by capacity doubling (sfe_db_create allocates exactly `rows`); the tiles follow the capacity under the
+ * budget above, and are released when they no longer fit it (a later many-query search may build them again). */
+int sfe_db_rows(const sfe_db *db, int64_t *rows); /* rows the next search sees */
+/* appends `rows` host rows (32 B each); *first_row (optional, host) = local row index of the first appended row */
+int sfe_db_append(sfe_matcher *m, sfe_db *db, const uint8_t *desc_host, int64_t rows, int64_t *first_row);
+/* appends from device memory of the matcher's device, in the extractor's cap-strided layout (sfe_stereo_frames_dev's
+ * desc_l and n_l): set i = rows [i*stride, i*stride + n_dev[i]) of desc_dev, appended in set order, rows in order.
+ * n_dev == NULL: every set holds `stride` rows (one contiguous block of count*stride rows). */
+int sfe_db_append_dev(sfe_matcher *m, sfe_db *db, const uint8_t *desc_dev, const int32_t *n_dev, int count, int stride,
+                      int64_t *first_row);
 /* out[q*4] = {idx0, dist0, idx1, dist1}: lexicographic (dist, idx) smallest two; -1/999999999
  * when the shard holds fewer rows.  The ratio test is (2*dist0 < dist1) on the caller's side. */
 int sfe_knn2(sfe_matcher *m, const sfe_db *db, const uint8_t *queries, int q, int32_t *out);

@@ -178,6 +178,9 @@ SIGNATURES = {
     "sfe_bowdb_query_dev": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _i]),
     "sfe_db_create": (_i, [_vp, _vp, _i64, _i64, _pp]),
     "sfe_db_destroy": (_i, [_vp]),
+    "sfe_db_rows": (_i, [_vp, C.POINTER(_i64)]),
+    "sfe_db_append": (_i, [_vp, _vp, _vp, _i64, C.POINTER(_i64)]),
+    "sfe_db_append_dev": (_i, [_vp, _vp, _vp, _vp, _i, _i, C.POINTER(_i64)]),
     "sfe_knn2": (_i, [_vp, _vp, _vp, _i, _vp]),
     "sfe_knn2_dev": (_i, [_vp, _vp, _vp, _i, _vp]),
     "sfe_knn2_merge_dev": (_i, [_vp, _vp, _i, _i, _vp]),
@@ -964,12 +967,39 @@ class BowDatabase:
 
 
 class DescriptorDB:
+    """A resident descriptor map searched by Matcher.knn2*: rows idx_base, idx_base + 1, ... in creation and append order.
+    Several matchers of the device may append to and search it from several threads."""
+
     def __init__(self, matcher: Matcher, desc, idx_base=0):
         desc = np.ascontiguousarray(desc, np.uint8)
         assert desc.ndim == 2 and desc.shape[1] == 32
         h = C.c_void_p()
         _check(lib().sfe_db_create(matcher.h, _p(desc), len(desc), idx_base, C.byref(h)))
-        self.h, self.rows, self.idx_base = h, len(desc), idx_base
+        self.m, self.h, self.rows, self.idx_base = matcher, h, len(desc), idx_base
+
+    def __len__(self):
+        n = C.c_int64()
+        _check(lib().sfe_db_rows(self.h, C.byref(n)))
+        return n.value
+
+    def append(self, desc, matcher=None) -> int:
+        """Appends host rows (n x 32 uint8) -> the local row index of the first."""
+        desc = np.ascontiguousarray(desc, np.uint8)
+        assert desc.ndim == 2 and desc.shape[1] == 32
+        first = C.c_int64()
+        _check(lib().sfe_db_append((matcher or self.m).h, self.h, _p(desc), len(desc), C.byref(first)))
+        self.rows = len(self)
+        return first.value
+
+    def append_dev(self, desc_ptr, n_ptr, count, stride, matcher=None) -> int:
+        """Appends `count` sets of rows held on the device in the extractor's cap-strided layout: set i = rows
+        [i * stride, i * stride + n[i]) of desc_ptr, n_ptr = device int32[count] (e.g. stereo_frames_dev's desc_l / n_l), or
+        None for `stride` rows per set -> the local row index of the first appended row."""
+        first = C.c_int64()
+        _check(lib().sfe_db_append_dev((matcher or self.m).h, self.h, _p(desc_ptr), _p(n_ptr), int(count), int(stride),
+                                       C.byref(first)))
+        self.rows = len(self)
+        return first.value
 
     def close(self):
         if getattr(self, "h", None):

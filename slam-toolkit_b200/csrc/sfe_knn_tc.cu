@@ -355,9 +355,11 @@ knn2_tc_kernel(const uint8_t *__restrict__ db, long long rows, long long idx_bas
 
 // Database rows -> ready-made operand tiles: tile t = rows 128 t .. 128 t + 127 as int8 {0, 1} in the K-major core-matrix layout
 // the MMA reads (32 KB per tile, 256 B per row: 8 x the packed map; rows past the end are zeros, which the epilogue never keys).
-__global__ void __launch_bounds__(256) knn2_unpack_tiles_kernel(const uint8_t *__restrict__ db, long long rows, uint8_t *__restrict__ tiles) {
-    const long long t0 = (long long)blockIdx.x * kTileN;
-    uint8_t *dst = tiles + (size_t)blockIdx.x * kBTileBytes;
+__global__ void __launch_bounds__(256) knn2_unpack_tiles_kernel(const uint8_t *__restrict__ db, long long rows, long long first_tile,
+                                                                uint8_t *__restrict__ tiles) {
+    const long long t = first_tile + blockIdx.x;
+    const long long t0 = t * kTileN;
+    uint8_t *dst = tiles + (size_t)t * kBTileBytes;
     for (int u = threadIdx.x; u < kTileN * 16; u += 256) {
         const int row = u >> 4, chunk16 = u & 15;
         const long long gr = t0 + row;
@@ -370,9 +372,11 @@ size_t knn2_tc_smem_bytes() { return sizeof(TcSmemT<2>) + 128; }
 int knn2_tc_group_queries() { return kGroupQ; }  // queries per work item: the caller sizes its chunks with it
 size_t knn2_tc_tiles_bytes(long long rows) { return (size_t)((rows + kTileN - 1) / kTileN) * kBTileBytes; }
 
-cudaError_t launch_knn2_unpack_tiles(cudaStream_t st, const uint8_t *db, long long rows, uint8_t *tiles) {
-    const long long n = (rows + kTileN - 1) / kTileN;
-    if (n > 0) knn2_unpack_tiles_kernel<<<(unsigned)n, 256, 0, st>>>(db, rows, tiles);
+// (re)writes tiles first_tile .. the one holding row rows - 1: 0 for a full build; an append into spare capacity starts at the
+// tile of its first new row, whose zero padding becomes real rows
+cudaError_t launch_knn2_unpack_tiles(cudaStream_t st, const uint8_t *db, long long rows, long long first_tile, uint8_t *tiles) {
+    const long long n = (rows + kTileN - 1) / kTileN - first_tile;
+    if (n > 0) knn2_unpack_tiles_kernel<<<(unsigned)n, 256, 0, st>>>(db, rows, first_tile, tiles);
     return cudaGetLastError();
 }
 

@@ -5,6 +5,7 @@
 #include <algorithm>
 #include <cmath>
 
+#include <functional>
 #include <mutex>
 
 #include "sfe_extract.cuh"
@@ -1201,6 +1202,58 @@ __global__ void __launch_bounds__(256) projection_gather_decode_kernel(CommView 
     if (dist) dist[j] = none ? -1 : (int32_t)(k >> 32);
 }
 
+// Descriptor-database append from device memory, part 1: off[i] = the rows of sets 0 .. i-1, off[count] = their total, or -1
+// when some n[i] lies outside [0, stride] (the host then appends nothing).  One CTA, a block-wide scan per 256 sets.
+__global__ void __launch_bounds__(256) db_append_offsets_kernel(const int32_t *__restrict__ n, int count, int stride,
+                                                                int64_t *__restrict__ off) {
+    __shared__ long long wsum[8];
+    __shared__ int bad;
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    if (t == 0) bad = 0;
+    __syncthreads();
+    long long base = 0;
+    for (int i0 = 0; i0 < count; i0 += 256) {
+        const int i = i0 + t;
+        long long own = 0;
+        if (i < count) {
+            const int c = n[i];
+            if (c < 0 || c > stride)
+                bad = 1;
+            else
+                own = c;
+        }
+        long long v = own;
+        for (int o = 1; o < 32; o <<= 1) {  // inclusive warp scan
+            const long long y = __shfl_up_sync(0xFFFFFFFFu, v, o);
+            if (lane >= o) v += y;
+        }
+        if (lane == 31) wsum[warp] = v;
+        __syncthreads();
+        long long before = 0, total = 0;
+        for (int w = 0; w < 8; w++) {
+            if (w < warp) before += wsum[w];
+            total += wsum[w];
+        }
+        if (i < count) off[i] = base + before + v - own;
+        base += total;
+        __syncthreads();
+    }
+    if (t == 0) off[count] = bad ? -1 : base;
+}
+
+// part 2: set i = rows [i * stride, i * stride + n[i]) of src -> rows off[i] .. of dst, one 16-byte word per thread and step.
+// Grid (chunks of a set, sets), both walked with the grid's stride.
+__global__ void __launch_bounds__(256) db_append_gather_kernel(const uint4 *__restrict__ src, const int32_t *__restrict__ n,
+                                                               const int64_t *__restrict__ off, int count, int stride,
+                                                               uint4 *__restrict__ dst) {
+    for (int i = blockIdx.y; i < count; i += gridDim.y) {
+        const long long words = 2ll * n[i];
+        const uint4 *s = src + 2ll * i * stride;
+        uint4 *d = dst + 2ll * off[i];
+        for (long long u = (long long)blockIdx.x * 256 + threadIdx.x; u < words; u += (long long)gridDim.x * 256) d[u] = __ldg(s + u);
+    }
+}
+
 }  // namespace sfe
 
 using namespace sfe;
@@ -1231,20 +1284,52 @@ struct sfe_matcher {
     DevBuf<unsigned long long> d_bow_chk;  // device vectors: nnz, rule broken, longest vector / assembly status
     DevBuf<int32_t> d_bowa_cnt, d_bowa_ids;  // BowVector assembly: words per set, vectors at the input's row stride,
     DevBuf<double> d_bowa_div, d_bowa_val;   // the divisor of each set's values
+    DevBuf<int64_t> d_db_off;      // descriptor-database appends from device memory: set offsets + total
+};
+
+// One event per stream that has read a resident database, recorded behind that read's kernels.  Whatever frees or rewrites
+// memory a queued read may still use waits for all of them first.  The database's lock guards it.
+struct ReaderEvents {
+    std::vector<std::pair<cudaStream_t, cudaEvent_t>> ev;
+    cudaError_t record(cudaStream_t st) {
+        for (auto &r : ev)
+            if (r.first == st) return cudaEventRecord(r.second, st);
+        cudaEvent_t e = nullptr;
+        cudaError_t err = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+        if (err != cudaSuccess) return err;
+        ev.emplace_back(st, e);
+        return cudaEventRecord(e, st);
+    }
+    cudaError_t sync() const {  // the host waits for every read enqueued so far
+        for (auto &r : ev) {
+            cudaError_t e = cudaEventSynchronize(r.second);
+            if (e != cudaSuccess) return e;
+        }
+        return cudaSuccess;
+    }
+    void release() {  // at destruction: wait, whatever the outcome, and destroy
+        for (auto &r : ev) {
+            cudaEventSynchronize(r.second);
+            cudaEventDestroy(r.second);
+        }
+        ev.clear();
+    }
 };
 
 struct sfe_db {
     int device = 0;
-    uint8_t *rows_dev = nullptr;
-    int64_t rows = 0, idx_base = 0;
-    // the rows as ready-made int8 operand tiles of the tensor-core kernel (8 x the packed size), built at the first
-    // many-query search when the policy (knn_tiles_max_bytes) allows; tiles_tried: do not try again.  Every matcher of the
-    // device may search the database, from any thread: tiles_mu guards the build, which runs on the stream of the matcher
-    // that comes first, and tiles_ready (recorded behind the unpack) is what every search that reads the tiles waits for.
-    mutable std::mutex tiles_mu;
+    uint8_t *rows_dev = nullptr;     // cap_rows rows; the first `rows` are the database
+    int64_t rows = 0, cap_rows = 0, idx_base = 0;
+    // the rows as ready-made int8 operand tiles of the tensor-core kernel (8 x the packed size, sized for cap_rows), built at
+    // the first many-query search when the policy (knn_tiles_max_bytes) allows; tiles_tried: do not try again.  An append
+    // keeps them current.  tiles_ready (recorded behind a search's build) is what every search that reads the tiles waits for.
     mutable uint8_t *tiles_dev = nullptr;
     mutable bool tiles_tried = false;
     mutable cudaEvent_t tiles_ready = nullptr;
+    // Every matcher of the device may append to and search the database, from any thread: mu guards everything above and
+    // `readers`.  A search reads rows_dev / rows / tiles_dev under it and records its stream's reader event behind its kernels.
+    mutable std::mutex mu;
+    mutable ReaderEvents readers;
 };
 
 // keys_out != nullptr: leave the per-keypoint (dist << 32 | ~global query) keys there (one shard's contribution to a
@@ -1340,13 +1425,29 @@ static int projection_impl(sfe_matcher *m, const double *xw, const uint8_t *mp_d
 namespace sfe {
 cudaError_t launch_knn2_tc(cudaStream_t st, int sm_count, const uint8_t *db, const uint8_t *tiles, long long rows, long long idx_base,
                            int chunk_rows, int chunks, const uint8_t *queries, int q, unsigned long long *part);
-cudaError_t launch_knn2_unpack_tiles(cudaStream_t st, const uint8_t *db, long long rows, uint8_t *tiles);
+cudaError_t launch_knn2_unpack_tiles(cudaStream_t st, const uint8_t *db, long long rows, long long first_tile, uint8_t *tiles);
 size_t knn2_tc_tiles_bytes(long long rows);
 int knn2_tc_group_queries();
 }
 
-static int knn_partial(sfe_matcher *m, const sfe_db *db, const uint8_t *q_dev, int q, unsigned long long *keys_dev,
-                       int32_t *quad_dev, const CommView *push = nullptr) {
+// A tile buffer for cap_rows rows when it fits the budget (SFE_KNN_TILES_MAX_GB, default 16 GB, and a quarter of the free
+// memory), else nullptr.
+static uint8_t *db_alloc_tiles(const sfe_matcher *m, int64_t cap_rows) {
+    const size_t need = knn2_tc_tiles_bytes(cap_rows);
+    size_t free_b = 0, total_b = 0;
+    uint8_t *t = nullptr;
+    if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need <= m->knn_tiles_max_bytes && need <= free_b / 4) {
+        if (cudaMalloc((void **)&t, need) != cudaSuccess) {
+            cudaGetLastError();
+            t = nullptr;
+        }
+    }
+    return t;
+}
+
+// Enqueues a search of the database's current rows; the caller holds db->mu.
+static int knn_enqueue(sfe_matcher *m, const sfe_db *db, const uint8_t *q_dev, int q, unsigned long long *keys_dev,
+                       int32_t *quad_dev, const CommView *push) {
     cudaStream_t st = m->stream;
     // Below 256 queries the group of 512 is mostly padding: worth it only when the map is large enough to hide the set-up.
     if (m->knn_tc && q >= m->knn_tc_min_q && db->rows >= 1 && (q >= 256 || db->rows >= 65536)) {
@@ -1361,38 +1462,27 @@ static int knn_partial(sfe_matcher *m, const sfe_db *db, const uint8_t *q_dev, i
         SFE_CUDA(m->d_part.ensure((size_t)chunks * q * 2));
         // A map that is searched with many queries keeps its rows unpacked in HBM (256 B per row instead of 32): the kernel's
         // producers then move tiles with bulk copies instead of unpacking 10 M rows once per query group.  Built on first use,
-        // when it fits the budget (SFE_KNN_TILES_MAX_GB, default 16 GB and a quarter of the free memory).
+        // when it fits the budget (db_alloc_tiles), for the database's capacity so that appends can extend them in place.
         const uint8_t *tiles = nullptr;
-        {
-            std::lock_guard<std::mutex> lock(db->tiles_mu);
-            if (!db->tiles_dev && !db->tiles_tried && q >= 256 && db->rows >= 65536) {
-                db->tiles_tried = true;
-                const size_t need = knn2_tc_tiles_bytes(db->rows);
-                size_t free_b = 0, total_b = 0;
-                uint8_t *t = nullptr;
-                if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need <= m->knn_tiles_max_bytes && need <= free_b / 4) {
-                    if (cudaMalloc((void **)&t, need) != cudaSuccess) {
-                        cudaGetLastError();
-                        t = nullptr;
-                    }
+        if (!db->tiles_dev && !db->tiles_tried && q >= 256 && db->rows >= 65536) {
+            db->tiles_tried = true;
+            uint8_t *t = db_alloc_tiles(m, db->cap_rows);
+            if (t) {  // published only once the unpack and the event behind it are enqueued
+                cudaError_t e = db->tiles_ready ? cudaSuccess : cudaEventCreateWithFlags(&db->tiles_ready, cudaEventDisableTiming);
+                if (e == cudaSuccess) e = launch_knn2_unpack_tiles(st, db->rows_dev, db->rows, 0, t);
+                if (e == cudaSuccess) e = cudaEventRecord(db->tiles_ready, st);
+                if (e != cudaSuccess) {
+                    cudaFree(t);
+                    set_error("knn2 tile build: %s", cudaGetErrorString(e));
+                    return SFE_ERR_CUDA;
                 }
-                if (t) {  // published only once the unpack and the event behind it are enqueued
-                    cudaError_t e = db->tiles_ready ? cudaSuccess : cudaEventCreateWithFlags(&db->tiles_ready, cudaEventDisableTiming);
-                    if (e == cudaSuccess) e = launch_knn2_unpack_tiles(st, db->rows_dev, db->rows, t);
-                    if (e == cudaSuccess) e = cudaEventRecord(db->tiles_ready, st);
-                    if (e != cudaSuccess) {
-                        cudaFree(t);
-                        set_error("knn2 tile build: %s", cudaGetErrorString(e));
-                        return SFE_ERR_CUDA;
-                    }
-                    db->tiles_dev = t;
-                    m->launches++;
-                }
+                db->tiles_dev = t;
+                m->launches++;
             }
-            if (db->tiles_dev) {
-                SFE_CUDA(cudaStreamWaitEvent(st, db->tiles_ready, 0));  // the unpack may run on another matcher's stream
-                tiles = db->tiles_dev;
-            }
+        }
+        if (db->tiles_dev) {
+            SFE_CUDA(cudaStreamWaitEvent(st, db->tiles_ready, 0));  // the unpack may run on another matcher's stream
+            tiles = db->tiles_dev;
         }
         SFE_CUDA(launch_knn2_tc(st, m->sm_count, db->rows_dev, tiles, db->rows, db->idx_base, (int)chunk_rows, chunks, q_dev, q,
                                 m->d_part.p));
@@ -1434,6 +1524,17 @@ static int knn_partial(sfe_matcher *m, const sfe_db *db, const uint8_t *q_dev, i
     return SFE_OK;
 }
 
+// A search sees exactly the rows appended before it was called: it is enqueued under the database's lock, and the stream's
+// reader event behind it holds back any append that would free or rewrite what it reads.
+static int knn_partial(sfe_matcher *m, const sfe_db *db, const uint8_t *q_dev, int q, unsigned long long *keys_dev,
+                       int32_t *quad_dev, const CommView *push = nullptr) {
+    std::lock_guard<std::mutex> lock(db->mu);
+    int rc = knn_enqueue(m, db, q_dev, q, keys_dev, quad_dev, push);
+    if (rc != SFE_OK) return rc;
+    SFE_CUDA(db->readers.record(m->stream));
+    return SFE_OK;
+}
+
 namespace sfe {
 cudaError_t launch_bow_score(cudaStream_t st, const int64_t *q_off, const int32_t *q_ids, const double *q_val, int q, int max_nq,
                              const int64_t *d_off, const int32_t *d_ids, const double *d_val, int n_entries, long long stride,
@@ -1457,9 +1558,8 @@ struct sfe_bowdb {
     int32_t *ids = nullptr;
     double *val = nullptr;
     mutable std::mutex mu;               // guards everything above and `readers`
-    // one event per stream that has queried the database, recorded behind that query's kernels: an add that outgrows the
-    // buffers waits for all of them before it frees the old ones
-    mutable std::vector<std::pair<cudaStream_t, cudaEvent_t>> readers;
+    // queries recorded behind their kernels: an add that outgrows the buffers waits for them before it frees the old ones
+    mutable ReaderEvents readers;
 };
 
 extern "C" {
@@ -1500,6 +1600,7 @@ int sfe_matcher_destroy(sfe_matcher *m) {
     m->d_bow_off.release(); m->d_bow_ids.release(); m->d_bow_e.release(); m->d_bow_n.release(); m->d_bow_val.release();
     m->d_bow_raw.release(); m->d_bow_dense.release(); m->d_bow_s.release(); m->d_bow_hit.release();
     m->d_bow_chk.release(); m->d_bowa_cnt.release(); m->d_bowa_div.release(); m->d_bowa_ids.release(); m->d_bowa_val.release();
+    m->d_db_off.release();
     cudaStreamDestroy(m->stream);
     delete m;
     return SFE_OK;
@@ -2113,10 +2214,7 @@ int sfe_bowdb_destroy(sfe_bowdb *db) {
     if (!db) return SFE_OK;
     DeviceGuard g(db->device);
     SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
-    for (auto &r : db->readers) {
-        cudaEventSynchronize(r.second);
-        cudaEventDestroy(r.second);
-    }
+    db->readers.release();
     cudaFree(db->off);
     if (db->ids) cudaFree(db->ids);
     if (db->val) cudaFree(db->val);
@@ -2141,7 +2239,7 @@ static int bow_reserve(sfe_bowdb *db, cudaStream_t st, int count, int64_t add_nn
     double *val = db->val;
     int64_t cap_e = db->cap_entries, cap_n = db->cap_nnz;
     if (need_e <= cap_e && need_nnz <= cap_n) return SFE_OK;
-    for (auto &r : db->readers) SFE_CUDA(cudaEventSynchronize(r.second));
+    SFE_CUDA(db->readers.sync());
     if (need_e > cap_e) cap_e = std::max(need_e, 2 * cap_e);
     if (need_nnz > cap_n) cap_n = std::max(need_nnz, 2 * cap_n);
     cudaError_t e = cudaSuccess;
@@ -2251,16 +2349,7 @@ static int bow_query_enqueue(sfe_matcher *m, const sfe_bowdb *db, const int64_t 
             SFE_CUDA(cudaMemcpy2DAsync(dense + (size_t)i0 * dense_entries, sizeof(double) * dense_entries, m->d_bow_dense.p,
                                        sizeof(double) * n_score, sizeof(double) * dense_entries, nb, dense_kind, st));
     }
-    cudaEvent_t *ev = nullptr;
-    for (auto &r : db->readers)
-        if (r.first == st) ev = &r.second;
-    if (!ev) {
-        cudaEvent_t e = nullptr;
-        SFE_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        db->readers.emplace_back(st, e);
-        ev = &db->readers.back().second;
-    }
-    SFE_CUDA(cudaEventRecord(*ev, st));
+    SFE_CUDA(db->readers.record(st));
     return SFE_OK;
 }
 
@@ -2367,7 +2456,7 @@ int sfe_db_create(sfe_matcher *m, const uint8_t *desc_host, int64_t rows, int64_
     SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
     sfe_db *db = new sfe_db();
     db->device = m->device;
-    db->rows = rows;
+    db->rows = db->cap_rows = rows;
     db->idx_base = idx_base;
     cudaError_t e = cudaMalloc((void **)&db->rows_dev, std::max<size_t>((size_t)rows * 32, 32));
     if (e == cudaSuccess && rows > 0) e = cudaMemcpy(db->rows_dev, desc_host, (size_t)rows * 32, cudaMemcpyHostToDevice);
@@ -2385,11 +2474,117 @@ int sfe_db_destroy(sfe_db *db) {
     if (!db) return SFE_OK;
     DeviceGuard g(db->device);
     SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    db->readers.release();
     cudaFree(db->rows_dev);
     if (db->tiles_dev) cudaFree(db->tiles_dev);
     if (db->tiles_ready) cudaEventDestroy(db->tiles_ready);
     delete db;
     return SFE_OK;
+}
+
+int sfe_db_rows(const sfe_db *db, int64_t *rows) {
+    SFE_REQUIRE(db && rows, SFE_ERR_BAD_ARG, "null argument");
+    std::lock_guard<std::mutex> lock(db->mu);
+    *rows = db->rows;
+    return SFE_OK;
+}
+
+// Appends `add` rows that put(dst) enqueues on the matcher's stream at dst = the first row past the database's end, under the
+// database's lock, and keeps the tiles current.  Synchronous; on failure the database keeps its rows.
+static int db_append_rows(sfe_matcher *m, sfe_db *db, int64_t add, int64_t *first_row,
+                          const std::function<cudaError_t(uint8_t *)> &put) {
+    cudaStream_t st = m->stream;
+    std::lock_guard<std::mutex> lock(db->mu);
+    const int64_t old = db->rows, rows = old + add;
+    SFE_REQUIRE(db->idx_base + rows < (1ll << 31), SFE_ERR_UNSUPPORTED, "global row index must fit int32");
+    if (add > 0 && rows <= db->cap_rows) {
+        // spare capacity: a queued search reads only rows below `old`, and of the tiles it may read only the one that holds
+        // row old - 1 is rewritten (its zero padding becomes real rows)
+        if (db->tiles_dev && old % 128 != 0) SFE_CUDA(db->readers.sync());
+        SFE_CUDA(put(db->rows_dev + (size_t)old * 32));
+        if (db->tiles_dev) {
+            SFE_CUDA(launch_knn2_unpack_tiles(st, db->rows_dev, rows, old / 128, db->tiles_dev));
+            m->launches++;
+        }
+        SFE_CUDA(cudaStreamSynchronize(st));
+    } else if (add > 0) {
+        // growth by capacity doubling: an append costs amortised O(its own size).  The old buffers are freed once every
+        // queued search has run.
+        SFE_CUDA(db->readers.sync());
+        const int64_t cap = std::max(rows, 2 * db->cap_rows);
+        uint8_t *r = nullptr;
+        cudaError_t e = cudaMalloc((void **)&r, (size_t)cap * 32);
+        if (e == cudaSuccess && old > 0) e = cudaMemcpyAsync(r, db->rows_dev, (size_t)old * 32, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = put(r + (size_t)old * 32);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) {
+            if (r) cudaFree(r);
+            set_error("descriptor database growth: %s", cudaGetErrorString(e));
+            return SFE_ERR_CUDA;
+        }
+        cudaFree(db->rows_dev);
+        db->rows_dev = r;
+        db->cap_rows = cap;
+        // tiles for the new capacity under the first build's budget, or none (the producer-unpack path gives the same
+        // results); a later many-query search may try again
+        db->tiles_tried = false;
+        if (db->tiles_dev) {
+            cudaFree(db->tiles_dev);
+            db->tiles_dev = db_alloc_tiles(m, cap);
+            if (db->tiles_dev) {
+                e = launch_knn2_unpack_tiles(st, db->rows_dev, rows, 0, db->tiles_dev);
+                if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+                m->launches++;
+                if (e != cudaSuccess) {
+                    cudaFree(db->tiles_dev);
+                    db->tiles_dev = nullptr;
+                    set_error("knn2 tile build: %s", cudaGetErrorString(e));
+                    return SFE_ERR_CUDA;
+                }
+            }
+        }
+    }
+    db->rows = rows;
+    if (first_row) *first_row = old;
+    return SFE_OK;
+}
+
+int sfe_db_append(sfe_matcher *m, sfe_db *db, const uint8_t *desc_host, int64_t rows, int64_t *first_row) {
+    SFE_REQUIRE(m && db && desc_host && rows >= 0, SFE_ERR_BAD_ARG, "bad argument");
+    SFE_REQUIRE(db->device == m->device, SFE_ERR_BAD_ARG, "database lives on another device");
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    return db_append_rows(m, db, rows, first_row, [&](uint8_t *dst) {
+        return cudaMemcpyAsync(dst, desc_host, (size_t)rows * 32, cudaMemcpyHostToDevice, m->stream);
+    });
+}
+
+int sfe_db_append_dev(sfe_matcher *m, sfe_db *db, const uint8_t *desc_dev, const int32_t *n_dev, int count, int stride,
+                      int64_t *first_row) {
+    SFE_REQUIRE(m && db && desc_dev && count >= 0 && stride >= 1, SFE_ERR_BAD_ARG, "bad argument");
+    SFE_REQUIRE(((uintptr_t)desc_dev & 15) == 0, SFE_ERR_BAD_ARG, "desc_dev must be 16-byte aligned");
+    SFE_REQUIRE(db->device == m->device, SFE_ERR_BAD_ARG, "database lives on another device");
+    DeviceGuard g(m->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    cudaStream_t st = m->stream;
+    int64_t add = (int64_t)count * stride;
+    if (n_dev && count > 0) {  // the counts are checked and scanned on the device before anything changes
+        SFE_CUDA(m->d_db_off.ensure((size_t)count + 1));
+        db_append_offsets_kernel<<<1, 256, 0, st>>>(n_dev, count, stride, m->d_db_off.p);
+        m->launches++;
+        SFE_CUDA(cudaGetLastError());
+        SFE_CUDA(cudaMemcpyAsync(&add, m->d_db_off.p + count, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        SFE_CUDA(cudaStreamSynchronize(st));
+        SFE_REQUIRE(add >= 0, SFE_ERR_BAD_ARG, "a set's row count n_dev[i] lies outside [0, stride]");
+    }
+    return db_append_rows(m, db, add, first_row, [&](uint8_t *dst) {
+        if (!n_dev) return cudaMemcpyAsync(dst, desc_dev, (size_t)add * 32, cudaMemcpyDeviceToDevice, st);
+        const int chunks = (int)std::min<int64_t>(((int64_t)stride * 2 + 255) / 256, 1024);
+        db_append_gather_kernel<<<dim3(chunks, std::min(count, 65535)), 256, 0, st>>>((const uint4 *)desc_dev, n_dev, m->d_db_off.p,
+                                                                                        count, stride, (uint4 *)dst);
+        m->launches++;
+        return cudaGetLastError();
+    });
 }
 
 int sfe_knn2_dev(sfe_matcher *m, const sfe_db *db, const uint8_t *queries_dev, int q, uint64_t *keys_dev) {
