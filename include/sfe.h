@@ -327,7 +327,8 @@ int sfe_frame_search_nearest(sfe_matcher *m, const sfe_frame *f, const double *u
  * The vocabulary as TemplatedVocabulary::loadFromTextFile holds it (thirdparty/DBoW2/DBoW2/TemplatedVocabulary.h:
  * 1338-1421): node 0 = root, node i >= 1 has parent[i] < i, a flag is_leaf[i], a 32-byte descriptor and a weight; the
  * children of a node are the nodes naming it as parent, in id order; words are numbered over the flagged nodes in
- * id order.  L = the header's depth (the `nid` level is counted from it). */
+ * id order.  L = the header's depth (the `nid` level is counted from it).  A node may have at most 2^20 - 1 children
+ * (the descent ranks a node's children in 20 bits); a vocabulary with a wider node returns SFE_ERR_UNSUPPORTED. */
 int sfe_vocab_create(sfe_matcher *m, int n_nodes, const int32_t *parent, const uint8_t *is_leaf,
                      const uint8_t *desc /* n_nodes x 32 */, const double *weight, int L, sfe_vocab **out);
 int sfe_vocab_destroy(sfe_vocab *v);

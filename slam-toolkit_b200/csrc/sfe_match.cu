@@ -983,6 +983,8 @@ __global__ void search_nearest_kernel(KpGrid G, const sfe_keypoint *__restrict__
 // current node (256-bit Hamming, FORB.cpp:81-101), the warp takes the minimum of (distance, child rank) -- the
 // reference's strict < keeps the first child on ties -- and steps down until it reaches a node without children.
 // ---------------------------------------------------------------------------------------------
+constexpr int kVocabMaxChildren = (1 << 20) - 1;  // children per node: the rank travels in the low 20 bits of the key
+
 struct VocabDev {
     const int *child_start;   // n_nodes + 1
     const int *child_list;    // children in id order
@@ -1006,12 +1008,12 @@ __global__ void __launch_bounds__(256) vocab_transform_kernel(VocabDev V, const 
         if (nc == 0) break;  // isLeaf()
         ++level;
         uint32_t best = kNoKey;
-        for (int c0 = 0; c0 < nc; c0 += 32) {  // k <= 20 in DBoW2's text format, so one round
+        for (int c0 = 0; c0 < nc; c0 += 32) {  // one round per 32 children; ORBvoc.txt has k = 10, so one round
             uint32_t key = kNoKey;
             if (c0 + lane < nc) {
                 uint32_t b[8];
                 load_desc(V.desc + (size_t)V.child_list[s + c0 + lane] * 32, b);
-                key = (uint32_t)hamming8(a, b) << 20 | (uint32_t)(c0 + lane);
+                key = (uint32_t)hamming8(a, b) << 20 | (uint32_t)(c0 + lane);  // rank < 2^20: sfe_vocab_create checks nc
             }
             best = min(best, __reduce_min_sync(0xffffffffu, key));
         }
@@ -2019,6 +2021,8 @@ int sfe_vocab_create(sfe_matcher *m, int n_nodes, const int32_t *parent, const u
         SFE_REQUIRE(parent[i] >= 0 && parent[i] < i, SFE_ERR_BAD_ARG, "a node must follow its parent (loadFromTextFile order)");
         start[parent[i] + 1]++;
     }
+    for (int i = 0; i < n_nodes; i++)  // the descent's (distance, child rank) key keeps the rank in 20 bits
+        SFE_REQUIRE(start[i + 1] <= kVocabMaxChildren, SFE_ERR_UNSUPPORTED, "a vocabulary node has more than 2^20 - 1 children");
     for (int i = 0; i < n_nodes; i++) start[i + 1] += start[i];
     int words = 0;
     for (int i = 1; i < n_nodes; i++) {
