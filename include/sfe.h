@@ -202,6 +202,43 @@ int sfe_stereo_sequence_dev(sfe_extractor *ex, const uint8_t *left_dev, const ui
                             int32_t *stereo_idx_dev, int32_t *stereo_dist_dev, int32_t *track_idx_dev,
                             int32_t *track_dist_dev, int cap);
 
+/* The tracker's per-pair behaviour for sfe_stereo_sequence_plan[_dev] (src/pipeline.cpp:158-166 predicts a pose for every
+ * frame; src/posetracker.cpp:185-190 matches again at a wider radius when too few points were found -- SURVEY §3.2).
+ *   rt / se3: NULL, or `frames` motion priors in host memory.  Entry f (f >= 1) is the Tcw of pair (f-1, f): it takes frame
+ *             f-1's camera coordinates into frame f's, exactly what tp->rt / tp->se3 is for every pair in
+ *             sfe_stereo_sequence.  Entry 0 is ignored.  rt = frames x 12 doubles (row-major 3x4, evaluated like tp->rt);
+ *             se3 = sfe_se3[frames] (evaluated like g2o::SE3Quat, as tp->se3).  At most one of the two may be non-NULL; both
+ *             NULL = tp's prior for every pair.  The priors are read before the call returns, also by an asynchronous _dev
+ *             call.
+ *   retry_radius, retry_below: a pair whose first ProjectionMatch (radius tp->radius) leaves fewer than retry_below
+ *             keypoints of frame f matched (the size of the std::map ProjectionMatch returns) is matched again with the same
+ *             map points, the same prior and radius retry_radius, and the second result replaces the first.
+ *             retry_below = 0: no retry.  The reference tracker: 100.0 and 8 (the rule as SURVEY §3.2 records it; the
+ *             reference sources are not part of this tree).
+ * SFE_ERR_BAD_ARG, before anything is enqueued: plan == NULL, both rt and se3 set, a prior of entries 1..frames-1 that is
+ * not finite, retry_radius negative or NaN, retry_below < 0 -- besides everything sfe_stereo_sequence[_dev] rejects. */
+typedef struct sfe_track_plan {
+    const double *rt;
+    const sfe_se3 *se3;
+    double retry_radius;
+    int32_t retry_below;
+} sfe_track_plan;
+/* sfe_stereo_sequence[_dev] with the pair priors and the retry of `plan`; every other argument and output as there.  A plan
+ * with both priors NULL (or every prior equal to tp's) and retry_below = 0 gives exactly what sfe_stereo_sequence gives. */
+int sfe_stereo_sequence_plan(sfe_extractor *ex, const uint8_t *left, const uint8_t *right,
+                             size_t image_stride, int frames, int w, int h, int stride,
+                             const sfe_stereo_params *sp, const sfe_track_params *tp,
+                             const sfe_track_plan *plan, sfe_keypoint *kps_l, uint8_t *desc_l, int32_t *n_l,
+                             sfe_keypoint *kps_r, uint8_t *desc_r, int32_t *n_r, int32_t *stereo_idx,
+                             int32_t *stereo_dist, int32_t *track_idx, int32_t *track_dist, int cap);
+int sfe_stereo_sequence_plan_dev(sfe_extractor *ex, const uint8_t *left_dev, const uint8_t *right_dev,
+                                 size_t image_stride, int frames, int w, int h, int stride,
+                                 const sfe_stereo_params *sp, const sfe_track_params *tp,
+                                 const sfe_track_plan *plan, sfe_keypoint *kps_l_dev, uint8_t *desc_l_dev,
+                                 int32_t *n_l_dev, sfe_keypoint *kps_r_dev, uint8_t *desc_r_dev,
+                                 int32_t *n_r_dev, int32_t *stereo_idx_dev, int32_t *stereo_dist_dev,
+                                 int32_t *track_idx_dev, int32_t *track_dist_dev, int cap);
+
 /* Row pitch (bytes) the _dev entry points like best for resident images of width w: the smallest multiple
  * of 16 >= w.  With such a pitch, a 16-byte aligned base and an image stride that is a multiple of 16 the
  * kernels fetch level-0 tiles with TMA; any other layout is read with ordinary loads (same results). */

@@ -88,6 +88,31 @@ class TrackParams(C.Structure):
         return t
 
 
+class TrackPlan(C.Structure):
+    """sfe_track_plan: per-pair motion priors (rt: frames x 12 doubles, or se3: frames SE3 records; entry f is the Tcw of pair
+    (f-1, f), entry 0 unused; both NULL = the track params' prior) and the tracker's wide-radius retry."""
+    _fields_ = [("rt", C.POINTER(C.c_double)), ("se3", C.POINTER(SE3)), ("retry_radius", C.c_double),
+                ("retry_below", C.c_int32)]
+
+
+def _track_plan(frames, priors, retry_radius, retry_below):
+    """-> (TrackPlan, the array its pointer refers to).  priors: None, (F, 7) SE3 values or (F, 3, 4) / (F, 4, 4) matrices."""
+    plan = TrackPlan(None, None, 100.0 if retry_radius is None else float(retry_radius),
+                     0 if retry_below is None else int(retry_below))
+    if priors is None:
+        return plan, None
+    a = np.asarray(priors, np.float64)
+    if a.ndim == 2 and a.shape == (frames, 7):
+        a = np.ascontiguousarray(a)
+        plan.se3 = a.ctypes.data_as(C.POINTER(SE3))
+    elif a.ndim == 3 and a.shape[0] == frames and a.shape[1:] in ((3, 4), (4, 4)):
+        a = np.ascontiguousarray(a[:, :3, :4]).reshape(frames, 12)
+        plan.rt = a.ctypes.data_as(C.POINTER(C.c_double))
+    else:
+        raise ValueError(f"priors: expected ({frames}, 7), ({frames}, 3, 4) or ({frames}, 4, 4), got {a.shape}")
+    return plan, a
+
+
 # every symbol include/sfe.h declares: name -> (restype, argtypes)
 _vp, _i, _sz, _d, _i64 = C.c_void_p, C.c_int, C.c_size_t, C.c_double, C.c_int64
 _pp = C.POINTER(C.c_void_p)
@@ -126,6 +151,10 @@ SIGNATURES = {
     "sfe_results_unpack": (_i, [_vp, _sz, _i] + [_vp] * 10),
     "sfe_stereo_sequence": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, C.POINTER(StereoParams), C.POINTER(TrackParams)] + [_vp] * 10 + [_i]),
     "sfe_stereo_sequence_dev": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, C.POINTER(StereoParams), C.POINTER(TrackParams)] + [_vp] * 10 + [_i]),
+    "sfe_stereo_sequence_plan": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, C.POINTER(StereoParams), C.POINTER(TrackParams),
+                                      C.POINTER(TrackPlan)] + [_vp] * 10 + [_i]),
+    "sfe_stereo_sequence_plan_dev": (_i, [_vp, _vp, _vp, _sz, _i, _i, _i, _i, C.POINTER(StereoParams), C.POINTER(TrackParams),
+                                          C.POINTER(TrackPlan)] + [_vp] * 10 + [_i]),
     "sfe_image_pitch": (_i, [_i]),
     "sfe_extractor_set_async": (_i, [_vp, _i]),
     "sfe_extractor_wait": (_i, [_vp]),
@@ -463,10 +492,14 @@ class ORBextractor:
         self._wh = (w, h)
         return out
 
-    def stereo_sequence(self, left, right, track_params, out=None, stereo_params=None):
+    def stereo_sequence(self, left, right, track_params, out=None, stereo_params=None, priors=None, retry_radius=None,
+                        retry_below=None):
         """Tracking front end of a stereo sequence: stereo_frames + per frame f >= 1 the ProjectionMatch of frame f-1's
         stereo-triangulated keypoints into frame f (sfe_stereo_sequence).  out["track_idx"][f, j] = keypoint of frame
-        f-1 matched to keypoint j of frame f, or -1."""
+        f-1 matched to keypoint j of frame f, or -1.
+        priors / retry_radius (default 100.0) / retry_below (default 0): the pair priors and the wide-radius retry of
+        sfe_stereo_sequence_plan (priors[f] = Tcw of pair (f-1, f), as (F, 7) SE3 values or (F, 3, 4) / (F, 4, 4)
+        matrices); the tracker's own retry is retry_radius=100.0, retry_below=8."""
         left = np.ascontiguousarray(left, np.uint8)
         right = np.ascontiguousarray(right, np.uint8)
         f, h, w = left.shape
@@ -476,21 +509,32 @@ class ORBextractor:
             out = self.alloc_stereo_out(f, track=True)
         cap = self._out_cap(out["kps_l"].shape[1], w, h)
         sp = C.byref(stereo_params) if stereo_params is not None else None
-        _check(lib().sfe_stereo_sequence(self.h, _p(left), _p(right), w * h, f, w, h, w, sp, C.byref(track_params),
-                                         _p(out["kps_l"]), _p(out["desc_l"]), _p(out["n_l"]), _p(out["kps_r"]),
-                                         _p(out["desc_r"]), _p(out["n_r"]), _p(out["stereo_idx"]), _p(out["stereo_dist"]),
-                                         _p(out["track_idx"]), _p(out["track_dist"]), cap))
+        args = [_p(out["kps_l"]), _p(out["desc_l"]), _p(out["n_l"]), _p(out["kps_r"]), _p(out["desc_r"]), _p(out["n_r"]),
+                _p(out["stereo_idx"]), _p(out["stereo_dist"]), _p(out["track_idx"]), _p(out["track_dist"]), cap]
+        if priors is None and retry_radius is None and retry_below is None:
+            _check(lib().sfe_stereo_sequence(self.h, _p(left), _p(right), w * h, f, w, h, w, sp, C.byref(track_params), *args))
+        else:
+            plan, keep = _track_plan(f, priors, retry_radius, retry_below)  # keep: the priors array, alive until the call returns
+            _check(lib().sfe_stereo_sequence_plan(self.h, _p(left), _p(right), w * h, f, w, h, w, sp, C.byref(track_params),
+                                                  C.byref(plan), *args))
         self._wh = (w, h)
         return out
 
-    def stereo_sequence_dev(self, left_ptr, right_ptr, frames, w, h, ptrs, track_params, stereo_params=None, pitch=None):
-        """stereo_frames_dev + tracking; ptrs additionally holds "track_idx" / "track_dist" (frames x cap int32)."""
+    def stereo_sequence_dev(self, left_ptr, right_ptr, frames, w, h, ptrs, track_params, stereo_params=None, pitch=None,
+                            priors=None, retry_radius=None, retry_below=None):
+        """stereo_frames_dev + tracking; ptrs additionally holds "track_idx" / "track_dist" (frames x cap int32).
+        priors / retry_radius / retry_below as stereo_sequence (host arrays, read before the call returns)."""
         sp = C.byref(stereo_params) if stereo_params is not None else None
         pitch = pitch or w
-        _check(lib().sfe_stereo_sequence_dev(self.h, _p(left_ptr), _p(right_ptr), pitch * h, frames, w, h, pitch, sp,
-                                             C.byref(track_params), _p(ptrs["kps_l"]), _p(ptrs["desc_l"]), _p(ptrs["n_l"]),
-                                             _p(ptrs["kps_r"]), _p(ptrs["desc_r"]), _p(ptrs["n_r"]), _p(ptrs["stereo_idx"]),
-                                             _p(ptrs["stereo_dist"]), _p(ptrs["track_idx"]), _p(ptrs["track_dist"]), self.cap))
+        args = [_p(ptrs["kps_l"]), _p(ptrs["desc_l"]), _p(ptrs["n_l"]), _p(ptrs["kps_r"]), _p(ptrs["desc_r"]), _p(ptrs["n_r"]),
+                _p(ptrs["stereo_idx"]), _p(ptrs["stereo_dist"]), _p(ptrs["track_idx"]), _p(ptrs["track_dist"]), self.cap]
+        if priors is None and retry_radius is None and retry_below is None:
+            _check(lib().sfe_stereo_sequence_dev(self.h, _p(left_ptr), _p(right_ptr), pitch * h, frames, w, h, pitch, sp,
+                                                 C.byref(track_params), *args))
+        else:
+            plan, keep = _track_plan(frames, priors, retry_radius, retry_below)  # keep: the priors array, alive until the call returns
+            _check(lib().sfe_stereo_sequence_plan_dev(self.h, _p(left_ptr), _p(right_ptr), pitch * h, frames, w, h, pitch, sp,
+                                                      C.byref(track_params), C.byref(plan), *args))
         self._wh = (w, h)
 
     def alloc_stereo_out(self, frames, pinned=False, track=False):

@@ -2221,7 +2221,8 @@ constexpr int kGraphMaxImages = 8;  // host calls with at most this many images 
 static int run_host_batch_once(sfe_extractor *ex, const uint8_t *left, const uint8_t *right, size_t image_stride, int frames, int w,
                                int h, int stride, const sfe_stereo_params *sp, sfe_keypoint *kps_l, uint8_t *desc_l, int32_t *n_l,
                                sfe_keypoint *kps_r, uint8_t *desc_r, int32_t *n_r, int32_t *stereo_idx, int32_t *stereo_dist,
-                               int cap, const sfe_track_params *tp, int32_t *track_idx, int32_t *track_dist) {
+                               int cap, const sfe_track_params *tp, const sfe_track_plan *plan, int32_t *track_idx,
+                               int32_t *track_dist) {
     const bool stereo = right != nullptr;
     const int images = stereo ? 2 * frames : frames;
     int rc = join_tail(ex);  // an asynchronous resident call may still be matching on the side stream
@@ -2429,10 +2430,15 @@ static int run_host_batch_once(sfe_extractor *ex, const uint8_t *left, const uin
         // (sout already waits for every sub-batch), on the D2H stream's tail
         SFE_CUDA_DRAIN(ex->d_tidx.ensure((size_t)ex->max_images * cap));
         SFE_CUDA_DRAIN(ex->d_tdist.ensure((size_t)ex->max_images * cap));
-        if ((rc = launch_track_frames(sout, ex->device, ex->track, frames, cap, kl, dl, nl, kr, ex->d_sidx.p, *tp, ex->d_tidx.p,
-                                      ex->d_tdist.p)) != SFE_OK)
-            return drain(rc);
-        ex->launches += 3;
+        if (plan) {
+            rc = launch_track_frames_plan(sout, ex->device, ex->track, frames, cap, kl, dl, nl, kr, ex->d_sidx.p, *tp, *plan,
+                                          ex->d_tidx.p, ex->d_tdist.p, ex->launches);
+        } else {
+            rc = launch_track_frames(sout, ex->device, ex->track, frames, cap, kl, dl, nl, kr, ex->d_sidx.p, *tp, ex->d_tidx.p,
+                                     ex->d_tdist.p);
+            ex->launches += 3;
+        }
+        if (rc != SFE_OK) return drain(rc);
         SFE_CUDA_DRAIN(cudaMemcpyAsync(track_idx, ex->d_tidx.p, sizeof(int32_t) * F * cap, cudaMemcpyDeviceToHost, sout));
         if (track_dist) SFE_CUDA_DRAIN(cudaMemcpyAsync(track_dist, ex->d_tdist.p, sizeof(int32_t) * F * cap, cudaMemcpyDeviceToHost, sout));
     }
@@ -2479,12 +2485,12 @@ static int run_host_batch_once(sfe_extractor *ex, const uint8_t *left, const uin
 static int run_host_batch(sfe_extractor *ex, const uint8_t *left, const uint8_t *right, size_t image_stride, int frames, int w,
                           int h, int stride, const sfe_stereo_params *sp, sfe_keypoint *kps_l, uint8_t *desc_l, int32_t *n_l,
                           sfe_keypoint *kps_r, uint8_t *desc_r, int32_t *n_r, int32_t *stereo_idx, int32_t *stereo_dist,
-                          int cap, const sfe_track_params *tp = nullptr, int32_t *track_idx = nullptr,
-                          int32_t *track_dist = nullptr) {
+                          int cap, const sfe_track_params *tp = nullptr, const sfe_track_plan *plan = nullptr,
+                          int32_t *track_idx = nullptr, int32_t *track_dist = nullptr) {
     int rc = kStatusRerun;
     for (int attempt = 0; attempt < 3 && rc == kStatusRerun; attempt++)  // one re-run suffices: the first pass counted exactly
         rc = run_host_batch_once(ex, left, right, image_stride, frames, w, h, stride, sp, kps_l, desc_l, n_l, kps_r, desc_r, n_r,
-                                 stereo_idx, stereo_dist, cap, tp, track_idx, track_dist);
+                                 stereo_idx, stereo_dist, cap, tp, plan, track_idx, track_dist);
     if (rc == kStatusRerun) { set_error("FAST candidate buffers still overflow after two re-runs"); rc = SFE_ERR_CAPACITY; }
     return rc;
 }
@@ -2567,7 +2573,7 @@ int sfe_extractor_destroy(sfe_extractor *ex) {
     ex->d_cand.release(); ex->d_kpst.release(); ex->d_counts.release();
     ex->d_tiles.release(); ex->d_segs.release(); ex->d_xtab.release(); ex->d_ytab.release();
     ex->d_kps.release(); ex->d_nout.release(); ex->d_sidx.release(); ex->d_sdist.release(); ex->d_tidx.release(); ex->d_tdist.release();
-    ex->track.cell_start.release(); ex->track.order.release(); ex->track.valid.release(); ex->track.sxy.release(); ex->track.sdesc.release(); ex->track.best.release();
+    ex->track.release();
     for (int i = 0; i <= kNumStages; i++)
         if (ex->prof_ev[i]) cudaEventDestroy(ex->prof_ev[i]);
     for (int i = 0; i < kMaxChunks; i++) {
@@ -2705,9 +2711,9 @@ int sfe_extract(sfe_extractor *ex, const uint8_t *image, int w, int h, int strid
 
 static int stereo_frames_dev_once(sfe_extractor *ex, const uint8_t *left_dev, const uint8_t *right_dev, size_t image_stride,
                                   int frames, int w, int h, int stride, const sfe_stereo_params *sp, const sfe_track_params *tp,
-                                  sfe_keypoint *kps_l_dev, uint8_t *desc_l_dev, int32_t *n_l_dev, sfe_keypoint *kps_r_dev,
-                                  uint8_t *desc_r_dev, int32_t *n_r_dev, int32_t *stereo_idx_dev, int32_t *stereo_dist_dev,
-                                  int32_t *track_idx_dev, int32_t *track_dist_dev, int cap) {
+                                  const sfe_track_plan *plan, sfe_keypoint *kps_l_dev, uint8_t *desc_l_dev, int32_t *n_l_dev,
+                                  sfe_keypoint *kps_r_dev, uint8_t *desc_r_dev, int32_t *n_r_dev, int32_t *stereo_idx_dev,
+                                  int32_t *stereo_dist_dev, int32_t *track_idx_dev, int32_t *track_dist_dev, int cap) {
     int rc = prepare(ex, 2 * frames, w, h, stride, cap);
     if (rc != SFE_OK) return rc;
     if (!sp) sp = &k_default_stereo;
@@ -2739,7 +2745,7 @@ static int stereo_frames_dev_once(sfe_extractor *ex, const uint8_t *left_dev, co
     cudaStream_t sm = tail ? ex->aux[1] : ex->stream;
     if (!tail) {
         if ((rc = join_tail(ex)) != SFE_OK) return rc;
-    } else if (tp && ex->tail_pending && (size_t)frames * cap > ex->track.best.n) {
+    } else if (tp && ex->tail_pending && track_scratch_grows(ex->track, frames, cap, plan)) {
         SFE_CUDA(cudaStreamSynchronize(ex->aux[1]));  // the tracking scratch is about to grow under a running tail
     }
     if (tail) {
@@ -2752,7 +2758,13 @@ static int stereo_frames_dev_once(sfe_extractor *ex, const uint8_t *left_dev, co
     ex->prof_has_stereo = true;
     ex->launches++;
     SFE_CUDA(cudaGetLastError());
-    if (tp) {
+    if (tp && plan) {
+        if ((rc = launch_track_frames_plan(sm, ex->device, ex->track, frames, cap, kps_l_dev, desc_l_dev, n_l_dev, kps_r_dev,
+                                           stereo_idx_dev, *tp, *plan, track_idx_dev, track_dist_dev, ex->launches)) != SFE_OK)
+            return rc;
+        prof_mark(ex, 7);
+        ex->prof_has_track = true;
+    } else if (tp) {
         if ((rc = launch_track_frames(sm, ex->device, ex->track, frames, cap, kps_l_dev, desc_l_dev, n_l_dev, kps_r_dev,
                                       stereo_idx_dev, *tp, track_idx_dev, track_dist_dev)) != SFE_OK)
             return rc;
@@ -2769,35 +2781,51 @@ static int stereo_frames_dev_once(sfe_extractor *ex, const uint8_t *left_dev, co
     return finish_dev(ex, 2 * frames);
 }
 
+static int check_track_params(const sfe_track_params *tp, const int32_t *track_idx) {
+    SFE_REQUIRE(tp && track_idx, SFE_ERR_BAD_ARG, "null argument");
+    SFE_REQUIRE(tp->cam.width >= 1 && tp->cam.height >= 1 && tp->cam.fx != 0. && tp->cam.fy != 0., SFE_ERR_BAD_ARG, "bad camera");
+    SFE_REQUIRE(tp->radius >= 0. && tp->radius == tp->radius, SFE_ERR_BAD_ARG, "bad radius");
+    return SFE_OK;
+}
+
+// a plan's contents, once `frames` is known to be valid (its priors are read for entries 1..frames-1)
+static int check_track_plan(const sfe_track_plan *plan, int frames) {
+    SFE_REQUIRE(!(plan->rt && plan->se3), SFE_ERR_BAD_ARG, "a track plan takes rt or se3 priors, not both");
+    SFE_REQUIRE(plan->retry_radius >= 0., SFE_ERR_BAD_ARG, "bad retry radius");
+    SFE_REQUIRE(plan->retry_below >= 0, SFE_ERR_BAD_ARG, "negative retry_below");
+    const int per = plan->rt ? 12 : 7;
+    const double *v = plan->rt ? plan->rt : plan->se3 ? &plan->se3->qx : nullptr;
+    static_assert(sizeof(sfe_se3) == 7 * sizeof(double), "sfe_se3 is read as 7 doubles");
+    for (size_t i = per; v && i < (size_t)frames * per; i++)
+        SFE_REQUIRE(std::isfinite(v[i]), SFE_ERR_BAD_ARG, "a motion prior is not finite");
+    return SFE_OK;
+}
+
 static int stereo_frames_dev_impl(sfe_extractor *ex, const uint8_t *left_dev, const uint8_t *right_dev, size_t image_stride,
                                   int frames, int w, int h, int stride, const sfe_stereo_params *sp, const sfe_track_params *tp,
-                                  sfe_keypoint *kps_l_dev, uint8_t *desc_l_dev, int32_t *n_l_dev, sfe_keypoint *kps_r_dev,
-                                  uint8_t *desc_r_dev, int32_t *n_r_dev, int32_t *stereo_idx_dev, int32_t *stereo_dist_dev,
-                                  int32_t *track_idx_dev, int32_t *track_dist_dev, int cap) {
+                                  const sfe_track_plan *plan, sfe_keypoint *kps_l_dev, uint8_t *desc_l_dev, int32_t *n_l_dev,
+                                  sfe_keypoint *kps_r_dev, uint8_t *desc_r_dev, int32_t *n_r_dev, int32_t *stereo_idx_dev,
+                                  int32_t *stereo_dist_dev, int32_t *track_idx_dev, int32_t *track_dist_dev, int cap) {
     SFE_REQUIRE(ex && left_dev && right_dev && kps_l_dev && desc_l_dev && n_l_dev && kps_r_dev && desc_r_dev && n_r_dev &&
                     stereo_idx_dev,
                 SFE_ERR_BAD_ARG, "null argument");
     SFE_REQUIRE(frames >= 1 && 2 * frames <= ex->max_images, SFE_ERR_BAD_ARG, "2*frames exceeds max_images");
+    if (plan)
+        if (int rc = check_track_plan(plan, frames)) return rc;
     DeviceGuard g(ex->device);
     SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
-    SFE_RERUN(stereo_frames_dev_once(ex, left_dev, right_dev, image_stride, frames, w, h, stride, sp, tp, kps_l_dev, desc_l_dev,
-                                     n_l_dev, kps_r_dev, desc_r_dev, n_r_dev, stereo_idx_dev, stereo_dist_dev, track_idx_dev,
-                                     track_dist_dev, cap));
+    SFE_RERUN(stereo_frames_dev_once(ex, left_dev, right_dev, image_stride, frames, w, h, stride, sp, tp, plan, kps_l_dev,
+                                     desc_l_dev, n_l_dev, kps_r_dev, desc_r_dev, n_r_dev, stereo_idx_dev, stereo_dist_dev,
+                                     track_idx_dev, track_dist_dev, cap));
 }
 
 int sfe_stereo_frames_dev(sfe_extractor *ex, const uint8_t *left_dev, const uint8_t *right_dev, size_t image_stride,
                           int frames, int w, int h, int stride, const sfe_stereo_params *sp, sfe_keypoint *kps_l_dev,
                           uint8_t *desc_l_dev, int32_t *n_l_dev, sfe_keypoint *kps_r_dev, uint8_t *desc_r_dev,
                           int32_t *n_r_dev, int32_t *stereo_idx_dev, int32_t *stereo_dist_dev, int cap) {
-    return stereo_frames_dev_impl(ex, left_dev, right_dev, image_stride, frames, w, h, stride, sp, nullptr, kps_l_dev, desc_l_dev,
-                                  n_l_dev, kps_r_dev, desc_r_dev, n_r_dev, stereo_idx_dev, stereo_dist_dev, nullptr, nullptr, cap);
-}
-
-static int check_track_params(const sfe_track_params *tp, const int32_t *track_idx) {
-    SFE_REQUIRE(tp && track_idx, SFE_ERR_BAD_ARG, "null argument");
-    SFE_REQUIRE(tp->cam.width >= 1 && tp->cam.height >= 1 && tp->cam.fx != 0. && tp->cam.fy != 0., SFE_ERR_BAD_ARG, "bad camera");
-    SFE_REQUIRE(tp->radius >= 0. && tp->radius == tp->radius, SFE_ERR_BAD_ARG, "bad radius");
-    return SFE_OK;
+    return stereo_frames_dev_impl(ex, left_dev, right_dev, image_stride, frames, w, h, stride, sp, nullptr, nullptr, kps_l_dev,
+                                  desc_l_dev, n_l_dev, kps_r_dev, desc_r_dev, n_r_dev, stereo_idx_dev, stereo_dist_dev, nullptr,
+                                  nullptr, cap);
 }
 
 int sfe_stereo_sequence_dev(sfe_extractor *ex, const uint8_t *left_dev, const uint8_t *right_dev, size_t image_stride, int frames,
@@ -2806,9 +2834,21 @@ int sfe_stereo_sequence_dev(sfe_extractor *ex, const uint8_t *left_dev, const ui
                             uint8_t *desc_r_dev, int32_t *n_r_dev, int32_t *stereo_idx_dev, int32_t *stereo_dist_dev,
                             int32_t *track_idx_dev, int32_t *track_dist_dev, int cap) {
     if (int rc = check_track_params(tp, track_idx_dev)) return rc;
-    return stereo_frames_dev_impl(ex, left_dev, right_dev, image_stride, frames, w, h, stride, sp, tp, kps_l_dev, desc_l_dev,
-                                  n_l_dev, kps_r_dev, desc_r_dev, n_r_dev, stereo_idx_dev, stereo_dist_dev, track_idx_dev,
-                                  track_dist_dev, cap);
+    return stereo_frames_dev_impl(ex, left_dev, right_dev, image_stride, frames, w, h, stride, sp, tp, nullptr, kps_l_dev,
+                                  desc_l_dev, n_l_dev, kps_r_dev, desc_r_dev, n_r_dev, stereo_idx_dev, stereo_dist_dev,
+                                  track_idx_dev, track_dist_dev, cap);
+}
+
+int sfe_stereo_sequence_plan_dev(sfe_extractor *ex, const uint8_t *left_dev, const uint8_t *right_dev, size_t image_stride,
+                                 int frames, int w, int h, int stride, const sfe_stereo_params *sp, const sfe_track_params *tp,
+                                 const sfe_track_plan *plan, sfe_keypoint *kps_l_dev, uint8_t *desc_l_dev, int32_t *n_l_dev,
+                                 sfe_keypoint *kps_r_dev, uint8_t *desc_r_dev, int32_t *n_r_dev, int32_t *stereo_idx_dev,
+                                 int32_t *stereo_dist_dev, int32_t *track_idx_dev, int32_t *track_dist_dev, int cap) {
+    if (int rc = check_track_params(tp, track_idx_dev)) return rc;
+    SFE_REQUIRE(plan, SFE_ERR_BAD_ARG, "null track plan");
+    return stereo_frames_dev_impl(ex, left_dev, right_dev, image_stride, frames, w, h, stride, sp, tp, plan, kps_l_dev,
+                                  desc_l_dev, n_l_dev, kps_r_dev, desc_r_dev, n_r_dev, stereo_idx_dev, stereo_dist_dev,
+                                  track_idx_dev, track_dist_dev, cap);
 }
 
 int sfe_stereo_frames(sfe_extractor *ex, const uint8_t *left, const uint8_t *right, size_t image_stride, int frames, int w,
@@ -2835,7 +2875,24 @@ int sfe_stereo_sequence(sfe_extractor *ex, const uint8_t *left, const uint8_t *r
     DeviceGuard g(ex->device);
     SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
     return run_host_batch(ex, left, right, image_stride, frames, w, h, stride, sp ? sp : &k_default_stereo, kps_l, desc_l, n_l,
-                          kps_r, desc_r, n_r, stereo_idx, stereo_dist, cap, tp, track_idx, track_dist);
+                          kps_r, desc_r, n_r, stereo_idx, stereo_dist, cap, tp, nullptr, track_idx, track_dist);
+}
+
+int sfe_stereo_sequence_plan(sfe_extractor *ex, const uint8_t *left, const uint8_t *right, size_t image_stride, int frames, int w,
+                             int h, int stride, const sfe_stereo_params *sp, const sfe_track_params *tp, const sfe_track_plan *plan,
+                             sfe_keypoint *kps_l, uint8_t *desc_l, int32_t *n_l, sfe_keypoint *kps_r, uint8_t *desc_r,
+                             int32_t *n_r, int32_t *stereo_idx, int32_t *stereo_dist, int32_t *track_idx, int32_t *track_dist,
+                             int cap) {
+    SFE_REQUIRE(ex && left && right && kps_l && desc_l && n_l && kps_r && desc_r && n_r && stereo_idx, SFE_ERR_BAD_ARG,
+                "null argument");
+    if (int rc = check_track_params(tp, track_idx)) return rc;
+    SFE_REQUIRE(plan, SFE_ERR_BAD_ARG, "null track plan");
+    SFE_REQUIRE(frames >= 1 && 2 * frames <= ex->max_images, SFE_ERR_BAD_ARG, "2*frames exceeds max_images");
+    if (int rc = check_track_plan(plan, frames)) return rc;
+    DeviceGuard g(ex->device);
+    SFE_REQUIRE(g.ok, SFE_ERR_NO_DEVICE, "cannot select the handle's device");
+    return run_host_batch(ex, left, right, image_stride, frames, w, h, stride, sp ? sp : &k_default_stereo, kps_l, desc_l, n_l,
+                          kps_r, desc_r, n_r, stereo_idx, stereo_dist, cap, tp, plan, track_idx, track_dist);
 }
 
 int sfe_image_pitch(int w) { return w > 0 ? (int)align_up((size_t)w, 16) : 0; }

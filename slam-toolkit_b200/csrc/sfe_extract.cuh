@@ -139,14 +139,36 @@ void launch_stereo_match(cudaStream_t st, int frames, int cap, const sfe_keypoin
 
 // sequence tracking launch (sfe_match.cu), used by sfe_stereo_sequence on the extractor's stream: per-frame bucket grids,
 // GetDepth + ProjectionMatch of frame f-1's stereo points into frame f, decode.  3 launches.
+struct Pose;
 struct TrackScratch {
     DevBuf<int> cell_start, order, valid;
     DevBuf<double2> sxy;
     DevBuf<uint4> sdesc;
     DevBuf<unsigned long long> best;
+    // sfe_stereo_sequence_plan: the pair priors, the keys of the retry pass and which pairs took it
+    DevBuf<Pose> poses;
+    DevBuf<unsigned long long> best2;
+    DevBuf<int> redo;
+    void release() {
+        cell_start.release(); order.release(); valid.release(); sxy.release(); sdesc.release(); best.release();
+        poses.release(); best2.release(); redo.release();
+    }
 };
 int launch_track_frames(cudaStream_t st, int device, TrackScratch &T, int frames, int cap, const sfe_keypoint *kl, const uint8_t *dl,
                         const int32_t *nl, const sfe_keypoint *kr, const int32_t *sidx, const sfe_track_params &tp,
                         int32_t *track_idx, int32_t *track_dist);
+// the same with a validated plan: the priors are copied on `st` before the call returns; 3 launches, 5 with a retry
+// (grids, first pass, retry flags, retry pass, decode; 2 for a single frame), added to `launches`
+int launch_track_frames_plan(cudaStream_t st, int device, TrackScratch &T, int frames, int cap, const sfe_keypoint *kl,
+                             const uint8_t *dl, const int32_t *nl, const sfe_keypoint *kr, const int32_t *sidx,
+                             const sfe_track_params &tp, const sfe_track_plan &plan, int32_t *track_idx, int32_t *track_dist,
+                             int64_t &launches);
+// would this call's tracking reallocate a buffer of T?  (an asynchronous call must not free one under a running tail)
+inline bool track_scratch_grows(const TrackScratch &T, int frames, int cap, const sfe_track_plan *plan) {
+    const size_t fc = (size_t)frames * cap;
+    if (fc > T.best.n) return true;
+    if (!plan) return false;
+    return (size_t)frames > T.poses.n || (plan->retry_below > 0 && (fc > T.best2.n || (size_t)frames > T.redo.n));
+}
 
 }  // namespace sfe

@@ -532,6 +532,12 @@ __global__ void __launch_bounds__(128) proj_match_sorted_kernel(KpGrid G, ProjPa
     project_and_match(G, P, xw[3 * (size_t)i], xw[3 * (size_t)i + 1], xw[3 * (size_t)i + 2], a, idx_base + i, best);
 }
 
+__device__ __forceinline__ void decode_key(unsigned long long k, int j, int32_t *__restrict__ to_query, int32_t *__restrict__ dist) {
+    const bool none = k == ~0ull;
+    to_query[j] = none ? -1 : (int32_t)(0xFFFFFFFFu - (uint32_t)(k & 0xFFFFFFFFu));
+    if (dist) dist[j] = none ? -1 : (int32_t)(k >> 32);
+}
+
 // keys of `shards` map-point shards (shards x m) -> per keypoint the minimum (dist, -query) key, decoded
 __global__ void projection_decode_kernel(int m, int shards, const unsigned long long *__restrict__ best,
                                          int32_t *__restrict__ to_query, int32_t *__restrict__ dist) {
@@ -539,9 +545,7 @@ __global__ void projection_decode_kernel(int m, int shards, const unsigned long 
     if (j >= m) return;
     unsigned long long k = best[j];
     for (int s = 1; s < shards; s++) k = min(k, best[(size_t)s * m + j]);
-    const bool none = k == ~0ull;
-    to_query[j] = none ? -1 : (int32_t)(0xFFFFFFFFu - (uint32_t)(k & 0xFFFFFFFFu));
-    if (dist) dist[j] = none ? -1 : (int32_t)(k >> 32);
+    decode_key(k, j, to_query, dist);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -891,10 +895,10 @@ __global__ void __launch_bounds__(256) track_grids_kernel(TrackArrays A) {
     if (tid == 0) A.n_valid[f] = nv;
 }
 
-// thread = keypoint i of frame f - 1 (f = blockIdx.y + 1): GetDepth, then ProjectionMatch into frame f
-__global__ void __launch_bounds__(128) track_match_kernel(TrackArrays A, ProjParams P, double baseline,
-                                                          unsigned long long *__restrict__ best) {
-    const int f = blockIdx.y + 1, prev = f - 1, e = blockIdx.x * blockDim.x + threadIdx.x;
+// thread = keypoint i of frame f - 1: GetDepth, then ProjectionMatch into frame f
+__device__ __forceinline__ void track_match_pair(const TrackArrays &A, const ProjParams &P, int f, double baseline,
+                                                 unsigned long long *__restrict__ best) {
+    const int prev = f - 1, e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= A.n_valid[prev]) return;  // keypoints without a stereo correspondence have no depth, hence no map point
     const int i = A.valid[(size_t)prev * A.cap + e], j = A.sidx[(size_t)prev * A.cap + i];
     const sfe_keypoint kp = A.kl[(size_t)prev * A.cap + i];
@@ -906,6 +910,50 @@ __global__ void __launch_bounds__(128) track_match_kernel(TrackArrays A, ProjPar
     load_desc(A.dl + ((size_t)prev * A.cap + i) * 32, a);
     const KpGrid G = track_grid(A, f);
     project_and_match(G, P, __dmul_rn(nrm.x, Z), __dmul_rn(nrm.y, Z), Z, a, (uint32_t)i, best + (size_t)f * A.cap);
+}
+
+// pair f = blockIdx.y + 1, one prior P.T for every pair
+__global__ void __launch_bounds__(128) track_match_kernel(TrackArrays A, ProjParams P, double baseline,
+                                                          unsigned long long *__restrict__ best) {
+    track_match_pair(A, P, blockIdx.y + 1, baseline, best);
+}
+
+// pair f = blockIdx.y + 1 with its own prior poses[f]; the retry pass (redo != nullptr) matches only the pairs flagged there
+__global__ void __launch_bounds__(128) track_match_plan_kernel(TrackArrays A, ProjParams P, double baseline,
+                                                               const Pose *__restrict__ poses, const int *__restrict__ redo,
+                                                               unsigned long long *__restrict__ best) {
+    const int f = blockIdx.y + 1;
+    if (redo && !redo[f]) return;
+    if ((int)(blockIdx.x * blockDim.x + threadIdx.x) >= A.n_valid[f - 1]) return;  // before the prior is loaded
+    P.T = poses[f];
+    track_match_pair(A, P, f, baseline, best);
+}
+
+// one CTA per pair f = blockIdx.x + 1: redo[f] = the first pass left fewer than retry_below keypoints of frame f holding a
+// map point (ProjectionMatch's std::map size: the keys written after the conflict rule)
+__global__ void __launch_bounds__(256) track_retry_flags_kernel(TrackArrays A, const unsigned long long *__restrict__ best,
+                                                                int retry_below, int *__restrict__ redo) {
+    __shared__ int total;
+    const int f = blockIdx.x + 1, m = min(A.nl[f], A.cap);
+    const unsigned long long *b = best + (size_t)f * A.cap;
+    if (threadIdx.x == 0) total = 0;
+    __syncthreads();
+    int c = 0;
+    for (int j = threadIdx.x; j < m; j += 256) c += b[j] != ~0ull;
+    c = __reduce_add_sync(0xffffffffu, c);
+    if ((threadIdx.x & 31) == 0) atomicAdd(&total, c);
+    __syncthreads();
+    if (threadIdx.x == 0) redo[f] = total < retry_below;
+}
+
+// projection_decode_kernel over frames x cap keys, each pair from the pass that holds its final result
+__global__ void track_decode_plan_kernel(int fc, int cap, const int *__restrict__ redo, const unsigned long long *__restrict__ best,
+                                         const unsigned long long *__restrict__ best2, int32_t *__restrict__ to_query,
+                                         int32_t *__restrict__ dist) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= fc) return;
+    const int f = j / cap;
+    decode_key(f > 0 && redo[f] ? best2[j] : best[j], j, to_query, dist);
 }
 
 // ReprojectionFilter::GetOutlier's per-keypoint quantity (src/posetracker.cpp:106-137): the distance between keypoint i
@@ -1027,10 +1075,10 @@ __global__ void __launch_bounds__(256) vocab_transform_kernel(VocabDev V, const 
     }
 }
 
-int launch_track_frames(cudaStream_t st, int device, TrackScratch &T, int frames, int cap, const sfe_keypoint *kl, const uint8_t *dl,
-                        const int32_t *nl, const sfe_keypoint *kr, const int32_t *sidx, const sfe_track_params &tp,
-                        int32_t *track_idx, int32_t *track_dist) {
-    TrackArrays A{};
+// scratch of a tracking call, the keys reset, the per-frame bucket grids enqueued (one launch)
+static int track_grids(cudaStream_t st, int device, TrackScratch &T, int frames, int cap, const sfe_keypoint *kl, const uint8_t *dl,
+                       const int32_t *nl, const sfe_keypoint *kr, const int32_t *sidx, const sfe_track_params &tp, TrackArrays &A) {
+    A = TrackArrays{};
     A.frames = frames; A.cap = cap;
     A.gw = (std::max(tp.cam.width, 1) >> kGridShift) + 1;
     A.gh = (std::max(tp.cam.height, 1) >> kGridShift) + 1;
@@ -1055,15 +1103,69 @@ int launch_track_frames(cudaStream_t st, int device, TrackScratch &T, int frames
     }
     SFE_CUDA(cudaMemsetAsync(T.best.p, 0xFF, sizeof(unsigned long long) * fc, st));
     track_grids_kernel<<<frames, 256, smem, st>>>(A);
+    return SFE_OK;
+}
+
+static ProjParams track_proj_params(const sfe_track_params &tp) {
+    ProjParams P;
+    P.T = tp.use_se3 ? pose_from_se3(&tp.se3) : pose_from_rt(tp.rt);
+    P.cam = tp.cam;
+    P.radius = tp.radius;
+    P.ratio = tp.best12_threshold;
+    return P;
+}
+
+int launch_track_frames(cudaStream_t st, int device, TrackScratch &T, int frames, int cap, const sfe_keypoint *kl, const uint8_t *dl,
+                        const int32_t *nl, const sfe_keypoint *kr, const int32_t *sidx, const sfe_track_params &tp,
+                        int32_t *track_idx, int32_t *track_dist) {
+    TrackArrays A;
+    if (int rc = track_grids(st, device, T, frames, cap, kl, dl, nl, kr, sidx, tp, A)) return rc;
+    const size_t fc = (size_t)frames * cap;
+    if (frames > 1)
+        track_match_kernel<<<dim3(div_up(cap, 128), frames - 1), 128, 0, st>>>(A, track_proj_params(tp), tp.baseline, T.best.p);
+    projection_decode_kernel<<<div_up((int)fc, 256), 256, 0, st>>>((int)fc, 1, T.best.p, track_idx, track_dist);
+    SFE_CUDA(cudaGetLastError());
+    return SFE_OK;
+}
+
+int launch_track_frames_plan(cudaStream_t st, int device, TrackScratch &T, int frames, int cap, const sfe_keypoint *kl,
+                             const uint8_t *dl, const int32_t *nl, const sfe_keypoint *kr, const int32_t *sidx,
+                             const sfe_track_params &tp, const sfe_track_plan &plan, int32_t *track_idx, int32_t *track_dist,
+                             int64_t &launches) {
+    TrackArrays A;
+    if (int rc = track_grids(st, device, T, frames, cap, kl, dl, nl, kr, sidx, tp, A)) return rc;
+    launches++;
+    const size_t fc = (size_t)frames * cap;
     if (frames > 1) {
-        ProjParams P;
-        P.T = tp.use_se3 ? pose_from_se3(&tp.se3) : pose_from_rt(tp.rt);
-        P.cam = tp.cam;
-        P.radius = tp.radius;
-        P.ratio = tp.best12_threshold;
-        track_match_kernel<<<dim3(div_up(cap, 128), frames - 1), 128, 0, st>>>(A, P, tp.baseline, T.best.p);
+        ProjParams P = track_proj_params(tp);
+        // the priors go through pageable memory, so the caller's arrays are consumed before this returns, and they are copied on
+        // the stream that runs the tracking kernels: behind every earlier reader of T.poses
+        std::vector<Pose> h(frames, P.T);
+        for (int f = 1; f < frames; f++) {
+            if (plan.rt) h[f] = pose_from_rt(plan.rt + 12 * (size_t)f);
+            else if (plan.se3) h[f] = pose_from_se3(plan.se3 + f);
+        }
+        SFE_CUDA(T.poses.ensure(frames));
+        SFE_CUDA(cudaMemcpyAsync(T.poses.p, h.data(), sizeof(Pose) * frames, cudaMemcpyHostToDevice, st));
+        const dim3 grid(div_up(cap, 128), frames - 1);
+        track_match_plan_kernel<<<grid, 128, 0, st>>>(A, P, tp.baseline, T.poses.p, nullptr, T.best.p);
+        launches++;
+        if (plan.retry_below > 0) {
+            SFE_CUDA(T.best2.ensure(fc));
+            SFE_CUDA(T.redo.ensure(frames));
+            track_retry_flags_kernel<<<frames - 1, 256, 0, st>>>(A, T.best.p, plan.retry_below, T.redo.p);
+            SFE_CUDA(cudaMemsetAsync(T.best2.p, 0xFF, sizeof(unsigned long long) * fc, st));
+            P.radius = plan.retry_radius;
+            track_match_plan_kernel<<<grid, 128, 0, st>>>(A, P, tp.baseline, T.poses.p, T.redo.p, T.best2.p);
+            track_decode_plan_kernel<<<div_up((int)fc, 256), 256, 0, st>>>((int)fc, cap, T.redo.p, T.best.p, T.best2.p, track_idx,
+                                                                           track_dist);
+            launches += 3;
+            SFE_CUDA(cudaGetLastError());
+            return SFE_OK;
+        }
     }
     projection_decode_kernel<<<div_up((int)fc, 256), 256, 0, st>>>((int)fc, 1, T.best.p, track_idx, track_dist);
+    launches++;
     SFE_CUDA(cudaGetLastError());
     return SFE_OK;
 }
